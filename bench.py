@@ -156,10 +156,12 @@ def run_reference(args, rank, world):
     for s in range(args.warmup + args.steps):
         step[0] = s
         t0 = time.perf_counter()
-        orc.render(n_blocks, events_filter=window_events)  # voice-shard replicas summed at the end
+        bus, _ = orc.render(n_blocks, events_filter=window_events)  # voice-shard replicas summed at the end
         dt = time.perf_counter() - t0
         if s >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, bus)
     ms = 1e3 * float(np.mean(times))
     value = voices * n_blocks * BLOCK / (ms / 1e3)
     sample = (f"{voices} voices x {sample_seconds:g} s of audio per step ({voices * n_blocks * BLOCK:.3g} voice-samples; the workload's "
@@ -208,6 +210,24 @@ def emit_json(line) -> None:
         sys.stdout.flush()
     else:
         os.write(_JSON_FD, data)
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(dirname, bus) -> None:
+    """--dump-outputs: the mix bus [n_blocks, outputs, block] of the last timed step as DIR/bus.npy (f32), so that two
+    builds can be compared output for output.  A bus larger than DUMP_LIMIT_BYTES is cut to a fixed, seeded sample of
+    whole blocks; their indices go to DIR/bus_blocks.npy (f64, exact for any block count)."""
+    os.makedirs(dirname, exist_ok=True)
+    bus = np.ascontiguousarray(bus, dtype=np.float32)
+    n_blocks = bus.shape[0]
+    keep = min(n_blocks, (DUMP_LIMIT_BYTES - 4096) // (bus[:1].nbytes + 8))  # + one f64 index per block, + .npy headers
+    if keep < n_blocks:
+        blocks = np.sort(np.random.Generator(np.random.PCG64(0)).choice(n_blocks, keep, replace=False))
+        bus = bus[blocks]
+        np.save(os.path.join(dirname, "bus_blocks.npy"), blocks.astype(np.float64))
+    np.save(os.path.join(dirname, "bus.npy"), bus)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -278,8 +298,9 @@ def attach_peer_bus(env, proc, n_blocks, want):
     return peer_bus, "peer"
 
 
-def measure(env, args, workload, voices, seconds, steps, warmup, want_peer=True, with_e2e=True, sample_clocks=False):
-    """Device-resident `value` (+ optionally e2e) of one workload on this run's GPUs."""
+def measure(env, args, workload, voices, seconds, steps, warmup, want_peer=True, with_e2e=True, sample_clocks=False, keep_output=False):
+    """Device-resident `value` (+ optionally e2e) of one workload on this run's GPUs.  keep_output: res["bus"] is the
+    mix bus of the last timed step, on the host."""
     from knaster_b200.multi_gpu import reduce_bus
 
     torch = env.torch
@@ -337,6 +358,8 @@ def measure(env, args, workload, voices, seconds, steps, warmup, want_peer=True,
            "ms_per_step": ms_per_step, "kern_ms": kern_ms, "red_ms": red_ms, "kern_launches": kern_launches, "launches": launches,
            "step_ms_sum": sum(step_ms), "clocks": clocks, "info": info, "build_s": build_s, "bus_mode": bus_mode, "chunks": chunks,
            "n_blocks": n_blocks, "step_frames": step_frames, "h2d": proc.last_upload_bytes()}
+    if keep_output:
+        res["bus"] = bus.cpu().numpy()  # before the e2e leg below: at N > 1 it renders into the same buffer
 
     # ---- e2e: through the C ABI with host buffers (rank-local; N>1: plus the bus sum)
     if with_e2e:
@@ -550,7 +573,11 @@ def main():
     ap.add_argument("--cpu-voices", type=int, default=4096)
     ap.add_argument("--cpu-seconds", type=float, default=4.0)
     ap.add_argument("--ref-seconds", type=float, default=1.0, help="--impl reference: audio seconds per step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the mix bus of the last timed step to DIR/bus.npy (f32; over 64 MB a seeded sample of whole blocks)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if not args.voices:
         args.voices = DEFAULT_VOICES[args.workload]
     sys.stdout.flush()
@@ -579,7 +606,10 @@ def main():
     # the NCCL reduce and the torch.cuda.Event timers all live on the same stream
     torch.cuda.set_stream(torch.cuda.Stream())
 
-    res = measure(env, args, args.workload, args.voices, args.seconds, args.steps, args.warmup, want_peer=args.bus == "peer", sample_clocks=True)
+    res = measure(env, args, args.workload, args.voices, args.seconds, args.steps, args.warmup, want_peer=args.bus == "peer", sample_clocks=True,
+                  keep_output=bool(args.dump_outputs) and rank == 0)
+    if args.dump_outputs and rank == 0:  # rank 0 holds the summed bus
+        dump_outputs(args.dump_outputs, res.pop("bus"))
     checks = {} if args.no_parity else parity_and_bus_check(env, args)
     peaks, peak_src = measured_peaks()
     others = None
