@@ -1688,13 +1688,36 @@ const char *fused_recipe_name(int recipe) {
 }
 // recipe 1: two lanes per voice while that still leaves at most one warp per SM sub-partition (148 x 4)
 bool fm_two_lanes(uint32_t n_voices) { return (n_voices + FM_VPW - 1) / FM_VPW <= 148u * 4u; }
+// recipe 4's form, read once from the environment: launch_fused runs it and sub_scan_applies accepts the block sizes its chunks tile
+struct ScanForm {
+    // Default: two warps per voice (render_sub_scan2, 64-frame chunks): 4.3 ms per 10 s step of 256 voices.  KGPU_SCAN_WARPS=1
+    // selects the one-warp kernels, kept for measurements: render_sub_scan_n (KGPU_SCAN_FPL=2, 5.0 ms) and render_sub_scan
+    // (KGPU_SCAN_FPL=1, 5.8 ms)
+    bool two_warps;
+    // KGPU_SCAN_FPL: frames per lane of render_sub_scan_n (2 or 4; anything else = render_sub_scan)
+    int fpl;
+    // KGPU_SCAN_PIPE=0: render_sub_scan's unpipelined form (pre-pass, then the frame-parallel half), kept for measurements
+    bool pipe;
+    uint32_t chunk_frames() const {
+        if (two_warps) return 2 * SCAN_CHUNK;                         // render_sub_scan2<.., 2>
+        return fpl == 2 || fpl == 4 ? fpl * SCAN_CHUNK : SCAN_CHUNK;  // render_sub_scan_n<.., fpl>, render_sub_scan
+    }
+};
+static const ScanForm &scan_form() {
+    static const ScanForm f = [] {
+        const char *w = getenv("KGPU_SCAN_WARPS"), *n = getenv("KGPU_SCAN_FPL"), *p = getenv("KGPU_SCAN_PIPE");
+        return ScanForm{!(w && *w == '1'), n && *n ? atoi(n) : 2, !(p && *p == '0')};
+    }();
+    return f;
+}
 // recipe 0 -> 4: a bank this small leaves most schedulers without a warp under one-lane-per-voice; one warp per voice
 // with the frames of a chunk across the lanes is faster up to ~1500 voices (measured, 10 s steps: 256 voices 6.7 ms against
-// 13.0, 1024 9.3 against 13.1, 2048 15.2 against 13.2; DESIGN.md section 3).  Chunks of 32 frames must tile the block grid, so
-// that a render is identical however it is split into launches.
+// 13.0, 1024 9.3 against 13.1, 2048 15.2 against 13.2; DESIGN.md section 3).  The kernels number their chunks from the start
+// of each launch, and which frames a chunk scans decides their last bits: the chunks of the form launch_fused runs must tile
+// the block grid, so that a render is identical however it is split into launches.  Other block sizes take render_sub_asr.
 bool sub_scan_applies(uint32_t n_voices, uint32_t block_size) {
     static const int force = [] { const char *e = getenv("KGPU_SUB_SCAN"); return e ? atoi(e) : -1; }(); // 0 never, 1 always (tests / measurements)
-    if (block_size % SCAN_CHUNK) return false;
+    if (block_size % scan_form().chunk_frames()) return false;
     if (force >= 0) return force != 0;
     return n_voices <= 1024;
 }
@@ -1722,14 +1745,9 @@ cudaError_t launch_fused(int recipe, const FusedArgs &a, cudaStream_t stream) {
     }
     if (recipe == 2) return launch_add_wt(a, stream);
     if (recipe == 4) {
-        // KGPU_SCAN_PIPE=0: the unpipelined form (pre-pass, then the frame-parallel half), kept for measurements
-        static const bool pipe = [] { const char *e = getenv("KGPU_SCAN_PIPE"); return !(e && *e == '0'); }();
-        // Default: two warps per voice (render_sub_scan2, 64-frame chunks): 4.3 ms per 10 s step of 256 voices.  KGPU_SCAN_WARPS=1
-        // selects the one-warp kernels, kept for measurements: render_sub_scan_n (KGPU_SCAN_FPL=2, 5.0 ms) and render_sub_scan
-        // (KGPU_SCAN_FPL=1, 5.8 ms)
-        static const bool two_warps = [] { const char *e = getenv("KGPU_SCAN_WARPS"); return !(e && *e == '1'); }();
-        // KGPU_SCAN_FPL: frames per lane of render_sub_scan_n (2 or 4; 1 = render_sub_scan below)
-        static const int fpl = [] { const char *e = getenv("KGPU_SCAN_FPL"); return e && *e ? atoi(e) : 2; }();
+        const ScanForm &form = scan_form();
+        const bool pipe = form.pipe, two_warps = form.two_warps;
+        const int fpl = form.fpl;
         if (!two_warps && fpl == 2) {
             if (a.n_taps) render_sub_scan_n<true, 2><<<a.n_voices, 32, 0, stream>>>(a);
             else render_sub_scan_n<false, 2><<<a.n_voices, 32, 0, stream>>>(a);

@@ -106,6 +106,7 @@ class AudioProcessor:
         self._push_events()
         self._started = True
         _ffi.check(self._lib.kgpu_render_block(self._plan))
+        self._last_render_frames = self.block_size()   # read_taps() returns this block's frames
 
     def run(self, inputs) -> None:
         """``AudioProcessor::run(&[&[F]])`` (processor.rs:119-141): one block, one slice of block_size samples per graph input."""

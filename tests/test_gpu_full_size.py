@@ -5,6 +5,7 @@ cores), bus and >= 64 sampled pre-mix voice taps compared sample by sample.
     configs[1]  additive, 4096 SinWt partials x 10 s      taps bit-identical (integer phase), bus <= 1e-5
     configs[2]  subtractive, 16 384 voices x 10 s         taps <= 1e-4 (IIR budget), bus <= 1e-5
     configs[2B] the same with Envelope segments           taps <= 1e-4, bus <= 1e-5
+    subtractive, 1024 voices x 10 s (render_sub_scan)    taps <= 1e-4, bus <= 1e-5
     configs[3]  FM, 8192 voices x 10 s                    carrier taps <= 1e-5 (oscillator budget), bus <= 1e-5
 
 Tolerances are the north star's (BASELINE.json); what is measured is printed and is far tighter.  Ten seconds
@@ -56,6 +57,13 @@ def test_config1_additive_4096_partials_10s():
 
 def test_config2_subtractive_16384_voices_10s():
     bus_err, tap_err, tail = full_size("subtractive", 16384, "render_sub_asr")
+    assert tap_err.max() <= 1e-4 and tail <= 1e-4
+    assert bus_err <= 1e-5
+
+
+def test_subtractive_1024_voices_10s_on_the_scan_kernel():
+    # the largest bank the time-parallel kernel takes: the scan re-associates the filter's sums, so the IIR budget, over 10 s
+    bus_err, tap_err, tail = full_size("subtractive", 1024, "render_sub_scan")
     assert tap_err.max() <= 1e-4 and tail <= 1e-4
     assert bus_err <= 1e-5
 

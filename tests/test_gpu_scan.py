@@ -18,8 +18,8 @@ pytestmark = pytest.mark.gpu
 SR = 48000
 
 
-def render(build, n_blocks, outputs=2, no_scan=False, bpl=0, taps=True):
-    graph, proc = AudioProcessor.new(0, outputs, AudioProcessorOptions(no_scan=no_scan))
+def render(build, n_blocks, outputs=2, no_scan=False, bpl=0, taps=True, block=64):
+    graph, proc = AudioProcessor.new(0, outputs, AudioProcessorOptions(block_size=block, no_scan=no_scan))
     ids = build(graph)
     if taps:
         for i in ids:
@@ -30,8 +30,8 @@ def render(build, n_blocks, outputs=2, no_scan=False, bpl=0, taps=True):
     return out, (proc.read_taps() if taps else None), proc
 
 
-def oracle(build, n_blocks, outputs=2):
-    g = Graph(0, outputs, 64, SR)
+def oracle(build, n_blocks, outputs=2, block=64):
+    g = Graph(0, outputs, block, SR)
     ids = build(g)
     orc = OracleProcessor(g, ring_buffer_size=1 << 22)
     for i in ids:
@@ -60,21 +60,36 @@ def test_scan_kernel_matches_the_oracle_and_the_lane_kernel():
 
 
 def test_scan_kernel_is_launch_split_invariant_and_equals_block_by_block():
+    # The scan kernel's chunks (64 frames) are numbered from each launch's first frame, and which frames a chunk scans decides
+    # their last bits: only block sizes the chunks tile take it, every other one the bit-exact render_sub_asr.  Either way the
+    # render must not depend on how it is cut into launches (7 blocks: an odd number of chunks at block size 64).
     def build(graph):
         return banks.subtractive_bank(graph, 96, 1.0, n_notes=6)
 
-    a, ta, proc = render(build, 750)
-    assert proc.info()["kernels"] == ["render_sub_scan"]
-    for bpl in (7, 100):
-        b, tb, _ = render(build, 750, bpl=bpl)
-        assert np.array_equal(a, b) and np.array_equal(ta, tb)
-    graph, p1 = AudioProcessor.new(0, 2, AudioProcessorOptions())
-    build(graph)
-    blocks = []
-    for _ in range(200):
-        p1.run_without_inputs()
-        blocks.append(p1.output_block())
-    assert np.array_equal(np.stack(blocks), a[:200])
+    for block in (32, 64, 96, 128, 192):
+        n_blocks = SR // block
+        a, ta, proc = render(build, n_blocks, block=block)
+        assert proc.info()["kernels"] == ["render_sub_scan" if block % 64 == 0 else "render_sub_asr"], f"block size {block}"
+        for bpl in (7, 100):
+            b, tb, _ = render(build, n_blocks, bpl=bpl, block=block)
+            assert np.array_equal(a, b) and np.array_equal(ta, tb), f"block size {block}, {bpl} blocks per launch"
+        graph, p1 = AudioProcessor.new(0, 2, AudioProcessorOptions(block_size=block))
+        for i in build(graph):
+            p1.add_tap(i, 0)
+        blocks, tap_blocks = [], []
+        for _ in range(12800 // block):
+            p1.run_without_inputs()
+            blocks.append(p1.output_block())
+            tap_blocks.append(p1.read_taps())
+        assert np.array_equal(np.stack(blocks), a[:len(blocks)]), f"block size {block}: block by block"
+        assert np.array_equal(np.concatenate(tap_blocks, axis=1), ta[:, :len(blocks) * block]), f"block size {block}: block by block"
+
+
+def test_scan_kernel_takes_banks_up_to_1024_voices():
+    for n_voices, kernel in ((1024, "render_sub_scan"), (1025, "render_sub_asr")):
+        graph, proc = AudioProcessor.new(0, 2, AudioProcessorOptions())
+        banks.subtractive_bank(graph, n_voices, 0.1, n_notes=1)
+        assert proc.info()["kernels"] == [kernel], n_voices
 
 
 def test_scan_kernel_all_filter_types_events_and_out_of_domain_parameters():
@@ -119,6 +134,79 @@ def test_scan_kernel_all_filter_types_events_and_out_of_domain_parameters():
     assert np.isfinite(ref_taps).all()
     assert err.max() <= 1e-4, f"voice {int(np.argmax(err.max(axis=1)))}: {err.max():.3e}"
     assert np.abs(out - ref).max() <= 1e-5 * max(1.0, float(np.abs(ref).max()))
+
+
+def test_scan_kernel_chunk_hand_off_edges():
+    # Where one 64-frame chunk hands its state to the next: events on a chunk's last and first frames (63 / 64, 127 / 128) and on
+    # the last frame of a launch, an EnvAsr attack that ends exactly on a chunk boundary, a release on a chunk's last frame, and
+    # launches of one chunk, of an odd and of an even number of chunks.  One voice has an event in every chunk: all of its chunks
+    # run in reference order, so its tap is the oracle's bit for bit.
+    n_blocks = 60
+    n_frames = n_blocks * 64
+    att = 128 / SR
+    assert np.float32(att) * np.float32(SR) == 128.0     # attack rate 2^-7: the ramp reaches 1 after exactly 128 frames
+
+    def at(f):
+        return kn.Seconds.from_samples(int(f), SR)
+
+    def build(graph):
+        ids = []
+        with graph.edit() as g:
+            def voice(freq, fc, q, a=0.01, r=0.05):
+                saw = g.push(kn.PolyBlep(kn.Waveform.Sawtooth, freq).precise_timing(8))
+                svf = g.push(kn.SvfFilter(kn.SvfFilterType.Low, fc, q, 0.0).precise_timing(8))
+                env = g.push(kn.EnvAsr(a, r).wr_mul(1.0 / 8).precise_timing(8))
+                sig = (saw >> svf) * env
+                sig.out([0, 0]).to_graph_out()
+                ids.append(sig._outputs[0][0])
+                return saw, env
+
+            saw, env = voice(110.0, 900.0, 2.0)                # events on both sides of the first chunk boundaries
+            env.param("t_restart").trig_at(at(0))
+            for f, hz in ((63, 220.0), (64, 330.0), (127, 165.0), (128, 247.0)):
+                saw.param("freq").set_at(hz, at(f))
+            env.param("t_release").trig_at(at(20 * 64 + 63))   # a release on a chunk's last frame
+            env.param("t_restart").trig_at(at(30 * 64))
+            saw, env = voice(82.0, 400.0, 5.0, a=att)           # attack from frame 128 to 255: sustains from chunk 4 on
+            env.param("t_restart").trig_at(at(128))
+            env.param("t_release").trig_at(at(40 * 64 + 63))
+            saw, env = voice(147.0, 2500.0, 0.7)                # events on the last frame of launches of 3, 4 and 7 blocks
+            env.param("t_restart").trig_at(at(0))
+            for f, hz in ((191, 196.0), (255, 147.0), (383, 294.0), (447, 131.0), (511, 175.0)):
+                saw.param("freq").set_at(hz, at(f))
+            env.param("t_release").trig_at(at(3 * 64 - 1))
+            env.param("t_restart").trig_at(at(4 * 64 - 1))
+            saw, env = voice(98.0, 1200.0, 1.0)                 # an event in every chunk: every chunk exact
+            for c in range(n_blocks):
+                f = 64 * c + (37 * c) % 64
+                if c % 2 == 0:
+                    env.param("t_restart").trig_at(at(f))
+                saw.param("freq").set_at(98.0 * (1 + c % 5), at(f))
+            saw, env = voice(55.0, 60.0, 8.0)                   # no event after the first: the scan's state crosses every launch
+            env.param("t_restart").trig_at(at(0))
+            saw, env = voice(73.0, 20000.0, 4.0)
+            env.param("t_restart").trig_at(at(64))
+            env.param("t_release").trig_at(at(127))
+            env.param("t_restart").trig_at(at(128))
+            env.param("t_release").trig_at(at(n_frames - 1))    # on the render's last frame
+        return ids
+
+    ref, ref_taps = oracle(build, n_blocks)
+    every = 3
+    scale = np.abs(ref_taps).max(axis=1)
+    assert scale.min() > 0.01 / 8
+    first = None
+    for bpl in (0, 1, 3, 4, 7):                             # one launch (60 chunks), 1, 3 (odd), 4 (even), 7
+        out, taps, proc = render(build, n_blocks, bpl=bpl)
+        assert proc.info()["kernels"] == ["render_sub_scan"]
+        assert np.array_equal(taps[every], ref_taps[every]), f"blocks per launch {bpl}"
+        err = np.abs(taps - ref_taps).max(axis=1) / scale
+        assert err.max() <= 1e-4, f"blocks per launch {bpl}, voice {int(np.argmax(err))}: {err.max():.3e}"
+        assert np.abs(out - ref).max() <= 1e-5
+        if first is None:
+            first = (out, taps)
+        else:
+            assert np.array_equal(out, first[0]) and np.array_equal(taps, first[1]), f"blocks per launch {bpl}"
 
 
 def test_small_bank_is_faster_on_the_scan_kernel():
