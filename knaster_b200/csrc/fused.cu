@@ -1319,7 +1319,17 @@ struct FmVoice {
         cph = cn > 1.0f ? cn - 1.0f : cn;
         return c * amp;
     }
-    KN_DEV bool inrange() const { return fabsf(moff) < 16.0f && fabsf(coff) < 16.0f && fabsf(mph) <= 2.0f && fabsf(cph) <= 2.0f; }
+    // Every sine argument of the next FM1_SUB frames stays below 120 (the branch-free restatement's domain): a phase moves by
+    // at most |increment| per frame (the wrap only brings a phase above 1 closer to 0), the modulator's increment is minc and
+    // the carrier's |v| / sr <= (|idx| + |fc|) / sr (|m| <= 1), and 18.5 * TAU = 116.2 leaves room for the roundings (and for
+    // rc_sr = div_prep(sr), which is within an ulp of 1 / sr: no division in the loop).
+    // Evaluated before every group: SinNumeric wraps its phase from above only, so at a negative frequency it descends
+    // without bound (osc.rs:266-268).
+    KN_DEV bool inrange(float rc_sr) const {
+        const float mspan = fabsf(mph) + fabsf(moff) + FM1_SUB * fabsf(minc);
+        const float cspan = fabsf(cph) + fabsf(coff) + FM1_SUB * ((fabsf(idx) + fabsf(fc)) * rc_sr);
+        return mspan < 18.5f && cspan < 18.5f;
+    }
 };
 
 template <bool TAPS>
@@ -1348,12 +1358,13 @@ __global__ void __launch_bounds__(32, 8) render_fm2_wide(FusedArgs a) {
             if (active && a.taps[i].voice == v) tap_row = (int)a.taps[i].tap;
 
     float *prow = a.partials + (size_t)(a.row0 + gwarp) * a.n_frames;
-    bool all_inrange = __all_sync(0xFFFFFFFFu, !active || s.inrange());
+    bool all_inrange = __all_sync(0xFFFFFFFFu, !active || s.inrange(rc_sr));
     for (uint32_t f0 = 0; f0 < a.n_frames; f0 += SUB_TILE) {
         const uint32_t nf = min((uint32_t)SUB_TILE, a.n_frames - f0);
 #pragma unroll 1
         for (uint32_t g0 = 0; g0 < SUB_TILE; g0 += FM1_SUB) {
             const uint32_t gf = f0 + g0;
+            all_inrange = __all_sync(0xFFFFFFFFu, !active || s.inrange(rc_sr));   // the phases have moved since the last group
             const bool ev_group = __any_sync(0xFFFFFFFFu, next_frame < gf + FM1_SUB);
             if (!ev_group && all_inrange && g0 + FM1_SUB <= nf) {
 #pragma unroll
@@ -1375,7 +1386,7 @@ __global__ void __launch_bounds__(32, 8) render_fm2_wide(FusedArgs a) {
                             next_frame = cur < end ? a.events[cur].frame : 0xFFFFFFFFu;
                             touched = true;
                         }
-                        if (__any_sync(0xFFFFFFFFu, touched)) all_inrange = __all_sync(0xFFFFFFFFu, !active || s.inrange());
+                        if (__any_sync(0xFFFFFFFFu, touched)) all_inrange = __all_sync(0xFFFFFFFFu, !active || s.inrange(rc_sr));
                         o = s.tick<false>(sr, rc_sr);
                         if (TAPS && tap_row >= 0) a.tap_out[(size_t)tap_row * a.tap_stride + a.tap_frame0 + gf + k] = o;
                     }
@@ -1471,9 +1482,13 @@ struct FmLane {
         }
         return arg;
     }
-    // |phase_offset| < 16 and |phase| <= 2: every sine argument is below 120 and the branch-free
-    // restatement of sinf applies
-    KN_DEV bool inrange() const { return fabsf(off) < 16.0f && fabsf(ph) <= 2.0f; }
+    // Every sine argument of this lane's next FM_SUB frames stays below 120, so the branch-free restatement of sinf applies
+    // (the bound of FmVoice::inrange: a carrier's increment is at most (|idx| + |fc|) / sr, a modulator's is inc; rc_sr ~ 1 / sr).
+    // Evaluated before every group: at a negative frequency the phase descends without bound.
+    KN_DEV bool inrange(float rc_sr) const {
+        const float step = car ? (fabsf(idx) + fabsf(fc)) * rc_sr : fabsf(inc);
+        return fabsf(ph) + fabsf(off) + FM_SUB * step < 18.5f;
+    }
 };
 
 template <bool TAPS>
@@ -1531,7 +1546,7 @@ __global__ void __launch_bounds__(32, 8) render_fm2(FusedArgs a) {
     bool q_ok = false;                                   // q[] holds the carrier increments of the next group (no numerator was tiny)
 #pragma unroll
     for (int k = 0; k < FM_SUB; k++) mcur[k] = q[k] = sn_old[k] = 0.f;
-    bool all_inrange = __all_sync(0xFFFFFFFFu, !active || s.inrange());
+    bool all_inrange = __all_sync(0xFFFFFFFFu, !active || s.inrange(rc_sr));
     uint32_t tile0 = 0;                                  // first frame of the staging tile the carriers are filling
     // steps (3): staging, exchange, increments of the next group.  Part of both branches below, so that the event-free one stays whole.
     auto hand_over = [&](uint32_t G, uint32_t gf) {
@@ -1567,6 +1582,7 @@ __global__ void __launch_bounds__(32, 8) render_fm2(FusedArgs a) {
         const uint32_t gf = G * FM_SUB;                  // the modulators' first frame in this iteration
         const uint32_t lf = gf - lag;                    // this lane's first frame (meaningful while role_on)
         const bool role_on = s.car ? (G >= 2 && G < NG + 2) : G < NG;
+        all_inrange = __all_sync(0xFFFFFFFFu, !active || s.inrange(rc_sr));       // the phases have moved since the last group
         const bool ev_group = __any_sync(0xFFFFFFFFu, role_on && next_frame < lf + FM_SUB);
         if (!ev_group && all_inrange && q_ok && G >= 3 && gf + FM_SUB <= NF) { // both roles have a whole group
             float arg[FM_SUB], sn_new[FM_SUB];
@@ -1606,7 +1622,7 @@ __global__ void __launch_bounds__(32, 8) render_fm2(FusedArgs a) {
                         next_frame = cur < end ? a.events[cur].frame : 0xFFFFFFFFu;
                         touched = true;
                     }
-                    if (__any_sync(0xFFFFFFFFu, touched)) all_inrange = __all_sync(0xFFFFFFFFu, !active || s.inrange());
+                    if (__any_sync(0xFFFFFFFFu, touched)) all_inrange = __all_sync(0xFFFFFFFFu, !active || s.inrange(rc_sr));
                     const float sn = kn_sinf(s.advance<false>(fm_pick(mcur, k), sr, rc_sr, valid));
                     // carriers: MathUGen<Mul> with the gain of this frame; modulators hand over the bare sample
                     fm_put(sn_new, k, s.car ? (valid && emit ? sn * s.amp : 0.f) : sn);

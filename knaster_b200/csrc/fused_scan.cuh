@@ -33,23 +33,7 @@
 
 constexpr int SCAN_CHUNK = 32;
 
-// The phase recurrence t' = wrap01(t + dt) is the longest dependent chain of a chunk: FADD -> compare -> FADD.  Two changes, both
-// with identical values:
-//   * rounding is monotone, so "fl(t + dt) >= 1" is the same predicate as "t >= T" for T = the smallest float whose sum with dt
-//     rounds to 1 or more -- a compare on the OLD phase, which issues beside the addition instead of behind it.  T is found by
-//     stepping from fl(1 - dt) one ulp at a time (at most a few steps); valid for dt in (0, 1), t in [0, 1), then T in [0.5, 1];
-//   * the 0/1 flag of that compare is made on the FMA pipe (4 cycles) instead of by FSET on the ALU pipe (~8): for t and T in
-//     [0.5, 1) both are multiples of 2^-24, so (t - T) * 2^24 + 1 is an integer, >= 1 exactly when t >= T and <= 0 otherwise; a
-//     smaller t only makes it more negative.  One FFMA.SAT (wrap_flag); the constant 1 - T * 2^24 is exact (|.| < 2^24).
-// Together: 8 cycles per frame instead of 16.
-KN_DEV float wrap_flag_const(float T) { return 1.0f - T * 16777216.0f; }
-KN_DEV float wrap_flag(float t, float c) { return __saturatef(__fmaf_rn(t, 16777216.0f, c)); }
-KN_DEV float wrap_threshold(float dt) {
-    float c = 1.0f - dt;
-    for (int i = 0; i < 4 && __fadd_rn(c, dt) >= 1.0f; i++) c = __uint_as_float(__float_as_uint(c) - 1u);
-    for (int i = 0; i < 8 && __fadd_rn(c, dt) < 1.0f; i++) c = __uint_as_float(__float_as_uint(c) + 1u);
-    return c;
-}
+// wrap_threshold, wrap_flag_const, wrap_flag (the phase recurrence's wrap as a compare on the old phase): csrc/nodes.cuh
 
 struct ScanK {
     float a[4];        // A, row-major

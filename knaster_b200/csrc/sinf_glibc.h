@@ -6,9 +6,10 @@
 // algorithm is the ARM optimized-routines sinf that glibc adopted in 2.28: sysdeps/ieee754/flt-32/
 // s_sinf.c + s_sincosf.h + s_sincosf_data.c).  This is a restatement of that published algorithm:
 // fast range reduction by pi/2 in f64 and a degree-7 sine / degree-8 cosine polynomial in f64,
-// rounded once to f32.  tests/test_host_plan.py::test_sinf_restatement_matches_libm checks it
-// bit-for-bit against the libm the oracle links, over millions of arguments in [-16, 16], and
-// tests/test_sinf_exhaustive.py (tools/sinf_exhaustive.cpp) over EVERY float below 120 in magnitude.
+// rounded once to f32; for |y| >= 120 glibc's reduce_large (y times 4/pi in integer arithmetic).  cosf is restated as well.
+// tests/test_host_plan.py::test_sinf_restatement_matches_libm checks the sine bit-for-bit against the libm the oracle
+// links, and tests/test_sinf_exhaustive.py (tools/sinf_exhaustive.cpp) both functions over EVERY float; the device
+// instantiation is checked over every float by tests/test_gpu_devmath.py (tools/devmath_exhaustive.cu).
 // The fused multiply-adds are glibc's too: on a CPU with FMA its ifunc selects __sinf_fma, the same source
 // compiled with contraction (12 of the 2.2e9 results differ from the un-fused build).
 //
@@ -19,9 +20,13 @@
 #include <string.h>
 #if defined(__CUDACC__)
 #define KN_SINF_HD __host__ __device__ __forceinline__
+// glibc's large-argument reduction is a call on the device (as the f64 sin / cos slow-path reduction was), with its quadrant
+// returned through memory as in glibc; the rest is inline
+#define KN_SINF_CALL __host__ __device__ inline __noinline__
 #else
 #include <cmath>
 #define KN_SINF_HD inline
+#define KN_SINF_CALL inline
 #endif
 
 namespace kgpu {
@@ -198,18 +203,104 @@ template <int N> __device__ __forceinline__ void kn_sinf_glibc_lean_n(const floa
 }
 #endif
 
-// Returns true and the sine in *out for |y| < 120 (glibc's reduce_fast domain); false otherwise
-// (the large-argument reduction is not restated).
-KN_SINF_HD bool kn_sinf_glibc(float y, float *out) {
-    uint32_t iy;
+// ---- the rest of glibc's sinf and all of its cosf (s_sinf.c, s_cosf.c) -----------------------------------------------------
+
+KN_SINF_HD uint32_t kn_f32_bits(float y) {
 #if defined(__CUDA_ARCH__)
-    iy = __float_as_uint(y);
+    return __float_as_uint(y);
 #else
-    memcpy(&iy, &y, 4);
+    uint32_t b;
+    memcpy(&b, &y, 4);
+    return b;
 #endif
-    if (((iy >> 20) & 0x7ff) >= 0x42f) return false;  // abstop12(120.0f)
-    *out = kn_sinf_glibc_inrange(y);
-    return true;
+}
+
+// sinf_poly: n even -> the sine polynomial, n odd -> the cosine polynomial, its coefficients negated when neg
+// (__sincosf_table[1]); fused operations as in __sinf_fma
+KN_SINF_HD float kn_sincosf_poly(double x, double x2, bool neg, int n) {
+    const double S1 = -0x1.555545995a603p-3, S2 = 0x1.1107605230bc4p-7, S3 = -0x1.994eb3774cf24p-13;
+    if ((n & 1) == 0) {
+        const double x3 = x * x2, s1 = kn_fma(x2, S3, S2), x7 = x3 * x2, s = kn_fma(x3, S1, x);
+        return (float)kn_fma(x7, s1, s);
+    }
+    const double g = neg ? -1.0 : 1.0; // sign changes are exact: the negated table's products and sums are the negated ones
+    const double C0 = g * 0x1p0, C1 = g * -0x1.ffffffd0c621cp-2, C2 = g * 0x1.55553e1068f19p-5, C3 = g * -0x1.6c087e89a359dp-10,
+                 C4 = g * 0x1.99343027bf8c3p-16;
+    const double x4 = x2 * x2, c2 = kn_fma(x2, C4, C3), c1 = kn_fma(x2, C1, C0), x6 = x4 * x2, c = kn_fma(x4, C2, c1);
+    return (float)kn_fma(x6, c2, c);
+}
+
+// glibc's __inv_pio4: 4/pi in overlapping 32-bit windows, one byte apart.  Constant memory on the device (a local array
+// would be stored to every kernel's stack at every call and cost the interpreter registers), a plain array on the host.
+#define KN_INV_PIO4                                                                                                              \
+    {0xa2,       0xa2f9,     0xa2f983,   0xa2f9836e, 0xf9836e4e, 0x836e4e44, 0x6e4e4415, 0x4e441529,                             \
+     0x441529fc, 0x1529fc27, 0x29fc2757, 0xfc2757d1, 0x2757d1f5, 0x57d1f534, 0xd1f534dd, 0xf534ddc0,                             \
+     0x34ddc0db, 0xddc0db62, 0xc0db6295, 0xdb629599, 0x6295993c, 0x95993c43, 0x993c4390, 0x3c439041}
+#if defined(__CUDACC__)
+static __constant__ const uint32_t kn_inv_pio4_dev[24] = KN_INV_PIO4;
+#endif
+#if !defined(__CUDA_ARCH__)
+static const uint32_t kn_inv_pio4_host[24] = KN_INV_PIO4;
+#endif
+#undef KN_INV_PIO4
+
+// glibc's reduce_large for 120 <= |y| < inf: y * 4/pi from 96 bits of 4/pi chosen by y's exponent, in integer arithmetic;
+// returns the reduced argument in radians and the quadrant in *np
+KN_SINF_CALL double kn_sincosf_reduce_large(uint32_t xi, int *np) {
+#if defined(__CUDA_ARCH__)
+    const uint32_t *arr = &kn_inv_pio4_dev[(xi >> 26) & 15];
+#else
+    const uint32_t *arr = &kn_inv_pio4_host[(xi >> 26) & 15];
+#endif
+    const double PI63 = 0x1.921FB54442D18p-62; // pi / 2^62
+    const int shift = (xi >> 23) & 7;
+    xi = ((xi & 0xffffff) | 0x800000) << shift;
+    uint64_t res0 = xi * arr[0];               // 32-bit product: only its low word is kept
+    const uint64_t res1 = (uint64_t)xi * arr[4], res2 = (uint64_t)xi * arr[8];
+    res0 = (res2 >> 32) | (res0 << 32);
+    res0 += res1;
+    const uint64_t n = (res0 + (1ULL << 61)) >> 62;
+    res0 -= n << 62;
+    *np = (int)n;
+    return (double)(int64_t)res0 * PI63;
+}
+
+// glibc's sinf (want_cos = false) or cosf (want_cos = true) for |y| >= 120: the large-argument path, whose sign table includes
+// y's sign.  +-inf and NaN give NaN (__math_invalidf).
+KN_SINF_HD float kn_sincosf_glibc_large(float y, bool want_cos) {
+    const uint32_t xi = kn_f32_bits(y);
+    if (((xi >> 20) & 0x7ff) >= 0x7f8) return y - y;
+    int n;
+    const double x = kn_sincosf_reduce_large(xi, &n);
+    const int q = (n + (int)(xi >> 31)) & 3;
+    const double s = (q == 1 || q == 2) ? -1.0 : 1.0; // sign[] = {1, -1, -1, 1}
+    return kn_sincosf_poly(x * s, x * x, (q & 2) != 0, want_cos ? n ^ 1 : n);
+}
+
+// glibc's sinf for every float: bit-identical to it (tools/sinf_exhaustive.cpp checks all 2^32 arguments)
+KN_SINF_HD float kn_sinf_glibc(float y) {
+    return ((kn_f32_bits(y) >> 20) & 0x7ff) < 0x42f ? kn_sinf_glibc_inrange(y) : kn_sincosf_glibc_large(y, false); // abstop12(120.0f)
+}
+
+// glibc's cosf for |y| < 120, straight-line like kn_sinf_glibc_inrange: for |y| < pi/4 the reduction gives n = 0 and leaves x
+// as it is, which is glibc's unreduced path; below 2^-12 the polynomial rounds to 1, glibc's special case
+KN_SINF_HD float kn_cosf_glibc_inrange(float y) { // requires |y| < 120
+    double x = (double)y;
+    const double r = x * 0x1.45F306DC9C883p+23;
+#if defined(__CUDA_ARCH__)
+    const int n = (__double2int_rz(r) + 0x800000) >> 24;
+#else
+    const int n = ((int32_t)r + 0x800000) >> 24;
+#endif
+    x = kn_fma(-(double)n, 0x1.921FB54442D18p0, x);
+    const int q = n & 3;
+    const double s = (q == 1 || q == 2) ? -1.0 : 1.0;
+    return kn_sincosf_poly(x * s, x * x, (q & 2) != 0, n ^ 1);
+}
+
+// glibc's cosf for every float
+KN_SINF_HD float kn_cosf_glibc(float y) {
+    return ((kn_f32_bits(y) >> 20) & 0x7ff) < 0x42f ? kn_cosf_glibc_inrange(y) : kn_sincosf_glibc_large(y, true);
 }
 
 } // namespace kgpu

@@ -343,7 +343,8 @@ def test_bad_events_are_reported_with_knaster_error_names():
 
 def test_sinf_restatement_matches_libm():
     """csrc/sinf_glibc.h (the device sine, host instantiation) against the libm the oracle links:
-    bit-for-bit over random + structured arguments in the domain SinNumeric / PolyBlep use."""
+    bit-for-bit over random + structured arguments in the domain SinNumeric / PolyBlep use, and over large ones
+    (a SinNumeric at a negative frequency or with a large phase offset reaches |x| >= 120)."""
     import ctypes.util
 
     lib = _ffi.lib()
@@ -358,13 +359,21 @@ def test_sinf_restatement_matches_libm():
         rng.uniform(-119.9, 119.9, 100_000),                     # whole reduce_fast domain
         np.float32(np.pi / 4) + np.arange(-2000, 2000) * np.float32(1e-7),
         np.logspace(-14, 0, 5000), [0.0, -0.0, 1e-30, 130.0, -500.0],
+        rng.uniform(-2.0 ** 20, -120.0, 100_000),                # glibc's reduce_large domain
+        rng.uniform(120.0, 2.0 ** 20, 100_000),
+        np.float32(120.0) + np.arange(-500, 500) * np.float32(2.0 ** -17),   # both sides of the path switch
+        -np.logspace(2.08, 38.5, 20_000), np.logspace(2.08, 38.5, 20_000),
+        [np.finfo(np.float32).max, -np.finfo(np.float32).max],
     ]).astype(np.float32)
     ys = np.empty_like(xs)
     _ffi.check(lib.kgpu_debug_sinf(xs.ctypes.data, ys.ctypes.data, len(xs)))
     ref = np.array([libm.sinf(float(x)) for x in xs], dtype=np.float32)
-    inside = np.abs(xs) < 120.0
-    assert np.array_equal(ys[inside].view(np.uint32), ref[inside].view(np.uint32))
-    assert np.abs(ys[~inside] - ref[~inside]).max() <= 1.2e-7   # fallback path: f64 sine rounded once
+    assert (np.abs(xs) >= 120.0).sum() > 200_000
+    assert np.array_equal(ys.view(np.uint32), ref.view(np.uint32))
+    special = np.array([np.inf, -np.inf, np.nan], dtype=np.float32)
+    ys = np.empty_like(special)
+    _ffi.check(lib.kgpu_debug_sinf(special.ctypes.data, ys.ctypes.data, len(special)))
+    assert np.isnan(ys).all()
 
 
 def test_event_calendar_does_not_change_what_the_device_sees():
