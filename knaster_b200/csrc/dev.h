@@ -28,7 +28,8 @@ enum DevKind : uint8_t {
     DK_PINK = 16,    // regs: 0,1 rng 2..10 white_noises[9] 11 always_on 12 counter(u32) 13 pink  noise.rs:53-115
     DK_BROWN = 17,   // regs: 0,1 rng 2 last_output                                        noise.rs:122-153
     DK_RANDLIN = 18, // regs: 0,1 rng 2 current_value 3 current_change_width 4 phase 5 phase_step  noise.rs:156-217
-    DK_PAN2 = 19,    // regs: 0 left_gain 1 right_gain (the host evaluates fast::cos / fast::sin when pan changes)  pan.rs:12-38
+    DK_PAN2 = 19,    // regs: 0 left_gain 1 right_gain (fast::cos / fast::sin of the pan position: evaluated by the host when a
+                     //       pan event arrives, by the kernel every frame while pan is routed at audio rate)  pan.rs:12-38
 };
 enum { REGS_SINWT = 3, REGS_SINNUM = 3, REGS_POLYBLEP = 5, REGS_SVF = 8, REGS_SVF_AR = 12, REGS_ONEPOLE = 3, REGS_ENV = 5,
        REGS_ENVELOPE_BASE = 8, REGS_ENVELOPE_PER_SEG = 6, REGS_CONST = 1, REGS_PHASOR = 4,
@@ -56,6 +57,10 @@ enum ArCode : uint8_t {
     // routes into an EnvAsr / EnvAr time: the rate is remade from the sample (idempotent, so the reference's "if changed" guard drops out)
     AR_ENV_ATTACK = 12,   // attack_rate = v == 0 ? 1 : 1 / (v * sr)    envelopes.rs:84-97,246-259
     AR_ENV_RELEASE = 13,  // release_rate likewise                       envelopes.rs:98-111,260-273
+    AR_PAN2_PAN = 14,     // pan2_gains(v * 0.5 + 0.5) -> left_gain, right_gain (fastapprox.h)   pan.rs:26-36
+    AR_PHASOR_FREQ = 15,  // step = (f64)v * (1 / (f64)sr)              osc.rs:191-197
+    AR_RANDLIN_FREQ = 16, // phase_step = v * (1 / sr) (f32)            noise.rs:206-213
+    AR_ENVELOPE_TIME_SCALE = 17, // step = (f64)v * (1 / (f64)sr)       envelopes.rs:477-479
     AR_POST = 32,         // AR_POST + k: value of arithmetic wrapper k = v (wr_mul)   math.rs:92-98
 };
 
@@ -63,7 +68,7 @@ constexpr int MAX_NODES = 24;   // nodes per voice template
 constexpr int MAX_IN = 8;       // MathUGen<N<=4>
 constexpr int MAX_OUT = 4;
 constexpr int MAX_POST = 3;
-constexpr int MAX_AR = 2;
+constexpr int MAX_AR = 6;       // every float parameter of a node: SvfFilter's three + one per WrMul (MAX_POST)
 constexpr int MAX_BUS = 8;      // graph outputs
 constexpr int MAX_REGS = 192;   // registers per voice
 constexpr int MAX_SLOTS = 24;   // live value slots per voice

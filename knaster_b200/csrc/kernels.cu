@@ -442,6 +442,7 @@ __global__ void __launch_bounds__(32) render_interp(InterpArgs a) {
                     }
                     return y;
                 };
+                const double isr = dn.n_ar ? 1.0 / (double)sr : 0.0; // (f64)(f32)sr is the integer rate: the host's 1 / sr exactly
                 FOR_GROUPS {
                     if (GROUP_PLAIN) {
                         PLAIN16(env_tick())
@@ -450,11 +451,14 @@ __global__ void __launch_bounds__(32) render_interp(InterpArgs a) {
                     for (uint32_t f = g0_; f < fe_; f++) {
                         EVENTS_AT(f, ENVL_STORE, ENVL_LOAD)
                         AR_POST_ROUTES(f)
+                        for (int ai = 0; ai < dn.n_ar; ai++) // envelopes.rs:477-479
+                            if (dn.ar_code[ai] == AR_ENVELOPE_TIME_SCALE) step = __dmul_rn((double)RDV(dn.ar_slot[ai], f), isr);
                         float y = env_tick();
                         EMIT(f, 0, y)
                     }
                 }
                 ENVL_STORE;
+                if (dn.n_ar) st_d(sreg, rb + 6, step);
                 break;
             }
             case DK_MATH: {
@@ -509,6 +513,7 @@ __global__ void __launch_bounds__(32) render_interp(InterpArgs a) {
             }
             case DK_PHASOR: {
                 double phase = ld_d(sreg, rb), step = ld_d(sreg, rb + 2);
+                const double isr = dn.n_ar ? 1.0 / (double)sr : 0.0;
                 FOR_GROUPS {
                     if (GROUP_PLAIN) {
                         PLAIN16(phasor_tick(phase, step))
@@ -517,11 +522,14 @@ __global__ void __launch_bounds__(32) render_interp(InterpArgs a) {
                     for (uint32_t f = g0_; f < fe_; f++) {
                         EVENTS_AT(f, st_d(sreg, rb, phase), (phase = ld_d(sreg, rb), step = ld_d(sreg, rb + 2)))
                         AR_POST_ROUTES(f)
+                        for (int ai = 0; ai < dn.n_ar; ai++) // osc.rs:191-197
+                            if (dn.ar_code[ai] == AR_PHASOR_FREQ) step = __dmul_rn((double)RDV(dn.ar_slot[ai], f), isr);
                         float y = phasor_tick(phase, step);
                         EMIT(f, 0, y)
                     }
                 }
                 st_d(sreg, rb, phase);
+                if (dn.n_ar) st_d(sreg, rb + 2, step);
                 break;
             }
             case DK_WHITE:
@@ -586,6 +594,7 @@ __global__ void __launch_bounds__(32) render_interp(InterpArgs a) {
                 uint64_t rng = ((uint64_t)sreg[(rb + 1) * 32] << 32) | sreg[rb * 32];
                 float cur = __uint_as_float(sreg[(rb + 2) * 32]), width = __uint_as_float(sreg[(rb + 3) * 32]),
                       phase = __uint_as_float(sreg[(rb + 4) * 32]), step = __uint_as_float(sreg[(rb + 5) * 32]);
+                const float isr = dn.n_ar ? 1.0f / sr : 0.0f;
                 FOR_GROUPS {
                     if (GROUP_PLAIN) {
                         PLAIN16(randlin_tick(rng, cur, width, phase, step))
@@ -594,6 +603,8 @@ __global__ void __launch_bounds__(32) render_interp(InterpArgs a) {
                     for (uint32_t f = g0_; f < fe_; f++) {
                         EVENTS_AT(f, (void)0, step = __uint_as_float(sreg[(rb + 5) * 32]))
                         AR_POST_ROUTES(f)
+                        for (int ai = 0; ai < dn.n_ar; ai++) // noise.rs:206-213
+                            if (dn.ar_code[ai] == AR_RANDLIN_FREQ) step = RDV(dn.ar_slot[ai], f) * isr;
                         float y = randlin_tick(rng, cur, width, phase, step);
                         EMIT(f, 0, y)
                     }
@@ -603,6 +614,7 @@ __global__ void __launch_bounds__(32) render_interp(InterpArgs a) {
                 sreg[(rb + 2) * 32] = __float_as_uint(cur);
                 sreg[(rb + 3) * 32] = __float_as_uint(width);
                 sreg[(rb + 4) * 32] = __float_as_uint(phase);
+                if (dn.n_ar) sreg[(rb + 5) * 32] = __float_as_uint(step);
                 break;
             }
             case DK_PAN2: { // pan.rs:31-36: [signal * left_gain, signal * right_gain]
@@ -611,10 +623,13 @@ __global__ void __launch_bounds__(32) render_interp(InterpArgs a) {
                 for (uint32_t f = 0; f < nf; f++) {
                     EVENTS_AT(f, (void)0, (gl = __uint_as_float(sreg[rb * 32]), gr = __uint_as_float(sreg[(rb + 1) * 32])))
                     AR_POST_ROUTES(f)
+                    for (int ai = 0; ai < dn.n_ar; ai++) // pan.rs:26-36: the gains of the routed pan position, every frame
+                        if (dn.ar_code[ai] == AR_PAN2_PAN) pan2_gains(RDV(dn.ar_slot[ai], f) * 0.5f + 0.5f, gl, gr);
                     const float x = RDV(is, f);
                     EMIT(f, 0, x * gl)
                     EMIT(f, 1, x * gr)
                 }
+                if (dn.n_ar) { sreg[rb * 32] = __float_as_uint(gl); sreg[(rb + 1) * 32] = __float_as_uint(gr); }
                 break;
             }
             case DK_CONST:

@@ -17,6 +17,7 @@
 //
 // Compiled with -ffp-contract=off: f32 expressions below must round exactly like rustc's.
 #include "plan.hpp"
+#include "fastapprox.h"
 
 #include <algorithm>
 #include <atomic>
@@ -83,33 +84,6 @@ inline float wy_f32(uint64_t &state) {
     float f;
     std::memcpy(&f, &bits, 4);
     return f - 1.0f;
-}
-
-// fastapprox 0.3.1 (fast::sin / fast::cos: Paul Mineiro's fastsin / fastcos), restated for Pan2 (pan.rs:31-36).
-// The crate is not under the reference tree: parity of these two functions is unpinned (DESIGN.md section 7).
-inline float fa_from_bits(uint32_t u) { float f; std::memcpy(&f, &u, 4); return f; }
-inline float fa_sin(float x) {
-    const float FOUROVERPI = 1.2732395447351627f, FOUROVERPISQ = 0.40528473456935109f, Q = 0.78444488374548933f;
-    uint32_t p = fbits(0.20363937680730309f), r = fbits(0.015124940802184233f), s = fbits(-0.0032225901625579573f);
-    uint32_t v = fbits(x);
-    const uint32_t sign = v & 0x80000000u;
-    v &= 0x7FFFFFFFu;
-    const float qpprox = FOUROVERPI * x - FOUROVERPISQ * x * fa_from_bits(v);
-    const float qpproxsq = qpprox * qpprox;
-    p |= sign;
-    r |= sign;
-    s ^= sign;
-    return Q * qpprox + qpproxsq * (fa_from_bits(p) + qpproxsq * (fa_from_bits(r) + qpproxsq * fa_from_bits(s)));
-}
-inline float fa_cos(float x) {
-    const float HALFPI = 1.5707963267948966f, HALFPIMINUSTWOPI = -4.7123889803846899f;
-    return fa_sin(x + (x > HALFPI ? HALFPIMINUSTWOPI : HALFPI));
-}
-// Pan2::process's two gains for a stored pan position (pan.rs:31-35)
-inline void pan2_gains(float pan01, float &gl, float &gr) {
-    const float rad = pan01 * 1.57079632679489661923f; // core::f32::consts::FRAC_PI_2
-    gl = fa_cos(rad);
-    gr = fa_sin(rad);
 }
 
 // ---- static facts about node kinds ------------------------------------------------------
@@ -635,6 +609,10 @@ uint8_t ar_code_for(const TemplateNode &tn, uint32_t param, int ar_level) {
         if (param == 0) return AR_ENV_ATTACK;
         if (param == 1) return AR_ENV_RELEASE;
         break; // the triggers are not floats: WrArParams would hand them a Float (a type error in knaster too)
+    case KGPU_PAN2: if (param == 0) return AR_PAN2_PAN; break;
+    case KGPU_PHASOR: if (param == 0) return AR_PHASOR_FREQ; break;
+    case KGPU_RANDOM_LIN: if (param == 0) return AR_RANDLIN_FREQ; break;
+    case KGPU_ENVELOPE: if (param == 0) return AR_ENVELOPE_TIME_SCALE; break; // jump_to_segment is an integer, the rest triggers
     default: break;
     }
     KGPU_THROW(KGPU_ERR_UNSUPPORTED, "audio-rate route to parameter %u of ugen kind %u is not supported yet", param, tn.kind);
