@@ -193,6 +193,88 @@ def chain_bank(graph: Graph, n_voices: int, seconds: float, seed: int = 5005, n_
     return out_ids
 
 
+def _notes(graph: Graph, env_ids: List[int], on: np.ndarray, off: np.ndarray, n_frames: int) -> None:
+    """EnvAsr notes: t_restart (3) at `on`, t_release (2) at `off`, any frame of a block."""
+    V, K = on.shape
+    env_a = np.repeat(np.asarray(env_ids, dtype=np.uint32), 2 * K).reshape(V, 2 * K)
+    frames = np.concatenate([on, off], axis=1)
+    params = np.concatenate([np.full((V, K), 3), np.full((V, K), 2)], axis=1)
+    order = np.argsort(frames, axis=1, kind="stable")
+    tk = lambda x: np.take_along_axis(x, order, 1).reshape(-1)
+    keep = tk(frames) < n_frames
+    n = int(keep.sum())
+    graph.schedule_bulk(tk(env_a)[keep], tk(params)[keep], np.full(n, 2), np.zeros(n), tk(frames)[keep].astype(np.uint64))
+
+
+def partials_bank(graph: Graph, n_voices: int, seconds: float, seed: int = 6006, n_partials: int = 32, n_notes: int = 4,
+                  voice_offset: int = 0, total_voices: int = 0) -> List[int]:
+    """A voice larger than 24 nodes: n_partials x SinWt(k f0).wr_mul(a_k) summed by an Add chain -> SvfFilter(Low) ->
+    * EnvAsr.wr_mul(1/N), note events (t_restart / t_release) at any frame.  32 partials = 66 nodes, 142 registers."""
+    total = total_voices or n_voices
+    sr = graph.sample_rate
+    n_frames = int(round(seconds * sr))
+    r = _rng(seed)
+    f0 = 55.0 * 2.0 ** r.uniform(0.0, 2.0, total)
+    amp = r.uniform(0.5, 1.0, (total, n_partials)) / np.arange(1, n_partials + 1) * 0.25
+    fc = r.uniform(500.0, 8000.0, total)
+    q = r.uniform(0.5, 4.0, total)
+    att = r.uniform(0.002, 0.05, total)
+    rel = r.uniform(0.05, 0.5, total)
+    on = np.sort(r.integers(0, max(1, n_frames), (total, n_notes)), axis=1)
+    off = on + (r.uniform(0.1, 0.4, (total, n_notes)) * sr).astype(np.int64)
+    sl = slice(voice_offset, voice_offset + n_voices)
+    f0, amp, fc, q, att, rel, on, off = (x[sl] for x in (f0, amp, fc, q, att, rel, on, off))
+    env_ids, out_ids = [], []
+    with graph.edit() as g:
+        for i in range(n_voices):
+            mix = None
+            for k in range(n_partials):
+                p = g.push(U.SinWt(float(f0[i] * (k + 1))).wr_mul(float(amp[i, k])))
+                mix = p if mix is None else mix + p
+            svf = g.push(U.SvfFilter(U.SvfFilterType.Low, float(fc[i]), float(q[i]), 0.0))
+            env = g.push(U.EnvAsr(float(att[i]), float(rel[i])).wr_mul(1.0 / total))
+            sig = (mix >> svf) * env
+            sig.out([0, 0]).to_graph_out()
+            env_ids.append(env.id()); out_ids.append(sig._outputs[0][0])
+    _notes(graph, env_ids, on, off, n_frames)
+    return out_ids
+
+
+def operator_bank(graph: Graph, n_voices: int, seconds: float, seed: int = 7007, n_ops: int = 12, n_notes: int = 4,
+                  voice_offset: int = 0, total_voices: int = 0) -> List[int]:
+    """A voice larger than 24 nodes made of builder arithmetic: PolyBlep(Sawtooth) -> n_ops x (x * a + b) -> SvfFilter(Low)
+    -> * EnvAsr.wr_mul(1/N), note events (t_restart / t_release) at any frame.  Each `x * a + b` pushes two Constants and two
+    MathUGens (graph_edit.rs:936-1225): 12 operators = 52 nodes."""
+    total = total_voices or n_voices
+    sr = graph.sample_rate
+    n_frames = int(round(seconds * sr))
+    r = _rng(seed)
+    f0 = 55.0 * 2.0 ** r.uniform(0.0, 4.0, total)
+    mul = r.uniform(0.9, 1.0, (total, n_ops))
+    add = r.uniform(-0.01, 0.01, (total, n_ops))
+    fc = r.uniform(500.0, 8000.0, total)
+    q = r.uniform(0.5, 4.0, total)
+    att = r.uniform(0.002, 0.05, total)
+    rel = r.uniform(0.05, 0.5, total)
+    on = np.sort(r.integers(0, max(1, n_frames), (total, n_notes)), axis=1)
+    off = on + (r.uniform(0.1, 0.4, (total, n_notes)) * sr).astype(np.int64)
+    sl = slice(voice_offset, voice_offset + n_voices)
+    f0, mul, add, fc, q, att, rel, on, off = (x[sl] for x in (f0, mul, add, fc, q, att, rel, on, off))
+    env_ids, out_ids = [], []
+    with graph.edit() as g:
+        for i in range(n_voices):
+            x = g.push(U.PolyBlep(U.Waveform.Sawtooth, float(f0[i])))
+            for k in range(n_ops):
+                x = x * float(mul[i, k]) + float(add[i, k])
+            svf = g.push(U.SvfFilter(U.SvfFilterType.Low, float(fc[i]), float(q[i]), 0.0))
+            env = g.push(U.EnvAsr(float(att[i]), float(rel[i])).wr_mul(1.0 / total))
+            sig = (x >> svf) * env
+            sig.out([0, 0]).to_graph_out()
+            env_ids.append(env.id()); out_ids.append(sig._outputs[0][0])
+    _notes(graph, env_ids, on, off, n_frames)
+    return out_ids
+
+
 def bank_builder(workload: str, seconds: float, seed=None):
     """The bench / parity workloads of BASELINE.json by name: returns build(graph, n_voices, voice_offset,
     total_voices) -> one tap node id per voice (the voice's pre-mix signal).  voice_offset / total_voices select a
@@ -209,6 +291,10 @@ def bank_builder(workload: str, seconds: float, seed=None):
             return fm_bank(graph, nv, voice_offset=offset, total_voices=total, **kw)
         if workload == "chain":
             return chain_bank(graph, nv, seconds, voice_offset=offset, total_voices=total, **kw)
+        if workload == "partials":
+            return partials_bank(graph, nv, seconds, voice_offset=offset, total_voices=total, **kw)
+        if workload == "operators":
+            return operator_bank(graph, nv, seconds, voice_offset=offset, total_voices=total, **kw)
         raise ValueError(f"unknown workload {workload}")
 
     return build

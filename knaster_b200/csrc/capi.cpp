@@ -186,11 +186,20 @@ namespace {
 // block size and whose value slots ([slot][chunk][32 lanes] f32) + registers fit 48 KB of shared memory.
 // A long chunk amortises what a node visit costs beside its arithmetic (dispatch, register load / store,
 // and above all instruction fetch: every node kind is its own block of code and a scheduler holds ONE warp).
-uint32_t pick_chunk(uint32_t block_size, uint32_t n_regs, uint32_t n_slots) {
-    uint32_t c = 64;
-    while (c > 1 && (block_size % c || ((size_t)n_regs + (size_t)n_slots * c) * 128 > 48 * 1024)) c >>= 1;
-    return c;
+// A template beyond the small-voice limits (dev.h) that gets fewer than 16 frames so goes up to 16 -- the length of the fast
+// paths' groups -- wherever the block size allows, in up to the 227 KB a block can opt into: (MAX_REGS + MAX_SLOTS * 16) * 128 B
+// fit.  Not more than 16: every kilobyte above 48 costs CTAs per SM, and a CTA is one warp.
+uint32_t pick_chunk(uint32_t block_size, const DevProgram &prog) {
+    auto fit = [&](uint32_t c, size_t budget) {
+        while (c > 1 && (block_size % c || ((size_t)prog.n_regs + (size_t)prog.n_slots * c) * 128 > budget)) c >>= 1;
+        return c;
+    };
+    const bool small = prog.n_nodes <= (uint32_t)SMALL_VOICE_NODES && prog.n_regs <= (uint32_t)SMALL_VOICE_REGS &&
+                       prog.n_slots <= (uint32_t)SMALL_VOICE_SLOTS;
+    const uint32_t c = fit(64, 48 * 1024);
+    return small || c >= 16 ? c : fit(16, 227 * 1024);
 }
+static_assert(((size_t)MAX_REGS + (size_t)MAX_SLOTS * 16) * 128 <= 227 * 1024, "a template inside the limits gets 16-frame chunks");
 
 void upload_program(kgpu_plan *p, uint32_t gi) {
     Group &g = p->host.groups[gi];
@@ -276,7 +285,7 @@ void choose_kernels(kgpu_plan *p) {
             else if (!err.empty()) p->jit_note = err;
         }
         d.recipe = recipe;
-        d.chunk = recipe >= 0 ? 1 : pick_chunk(p->host.block_size, g.prog.n_regs, g.prog.n_slots);
+        d.chunk = recipe >= 0 ? 1 : pick_chunk(p->host.block_size, g.prog);
         g.fused_recipe = recipe;
         g.kernel_name = recipe == RECIPE_JIT ? "render_jit" : recipe >= 0 ? fused_recipe_name(recipe) : "render_interp";
     }

@@ -64,14 +64,20 @@ enum ArCode : uint8_t {
     AR_POST = 32,         // AR_POST + k: value of arithmetic wrapper k = v (wr_mul)   math.rs:92-98
 };
 
-constexpr int MAX_NODES = 24;   // nodes per voice template
+// Per-voice limits.  A node index inside a template travels as a u8 on the host (RawEvent::local), so 128 nodes leave room;
+// the interpreter keeps registers and MAX_SLOTS x 16 frames of value slots of 32 lanes in shared memory:
+// (1024 + 32 * 16) * 128 B = 192 KB, under the 227 KB a block may opt into (capi.cpp pick_chunk).
+constexpr int MAX_NODES = 128;  // nodes per voice template
 constexpr int MAX_IN = 8;       // MathUGen<N<=4>
 constexpr int MAX_OUT = 4;
 constexpr int MAX_POST = 3;
 constexpr int MAX_AR = 6;       // every float parameter of a node: SvfFilter's three + one per WrMul (MAX_POST)
 constexpr int MAX_BUS = 8;      // graph outputs
-constexpr int MAX_REGS = 192;   // registers per voice
-constexpr int MAX_SLOTS = 24;   // live value slots per voice
+constexpr int MAX_REGS = 1024;  // registers per voice
+constexpr int MAX_SLOTS = 32;   // live value slots per voice
+// The limits before voices of up to MAX_NODES nodes: a template inside all three is "small".  Voice discovery keeps cutting
+// the graph where it did for such voices, and the interpreter keeps their chunk, so graphs that fitted them plan as before.
+constexpr int SMALL_VOICE_NODES = 24, SMALL_VOICE_REGS = 192, SMALL_VOICE_SLOTS = 24;
 
 struct DevNode {
     uint8_t kind, mode, n_in, n_out;

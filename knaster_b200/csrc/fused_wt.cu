@@ -215,8 +215,9 @@ bool match_add_wt(const DevProgram &p, uint32_t block_size) {
 }
 uint32_t add_wt_slices(uint32_t n_voices) { return std::max(1u, std::min(32u, (n_voices + 127) / 128)); }
 size_t add_wt_scratch_bytes(uint32_t n_voices, uint32_t n_frames, uint32_t block_size) {
-    // the per-(block, voice) records, then a second copy of the voice registers (see launch_add_wt)
-    return (size_t)n_voices * (n_frames / block_size) * sizeof(WtParam) + (size_t)n_voices * MAX_REGS * 4;
+    // the per-(block, voice) records, then a second copy of the voice registers (see launch_add_wt); the shape holds a few
+    // registers, far below the small-voice limit the copy is sized for
+    return (size_t)n_voices * (n_frames / block_size) * sizeof(WtParam) + (size_t)n_voices * SMALL_VOICE_REGS * 4;
 }
 cudaError_t launch_add_wt(const FusedArgs &a, cudaStream_t stream) {
     uint32_t gain_reg = 0xFFFFFFFFu;

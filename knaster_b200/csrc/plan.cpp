@@ -132,7 +132,7 @@ const char *param_types(uint32_t kind) {
 bool is_math_wrapper(uint32_t k) { return k >= KGPU_WR_MUL && k <= KGPU_WR_POWI; }
 
 void validate_node(const kgpu_node_desc &d, uint32_t idx) {
-    KindInfo ki = kind_info(d);
+    kind_info(d); // rejects an unknown kind
     if (d.kind == KGPU_MATH) {
         if (d.channels < 1 || d.channels > (uint32_t)MAX_OUT)
             KGPU_THROW(KGPU_ERR_UNSUPPORTED, "node %u: MathUGen with %u channels (1..%d supported)", idx, d.channels, MAX_OUT);
@@ -143,7 +143,9 @@ void validate_node(const kgpu_node_desc &d, uint32_t idx) {
     if (d.kind == KGPU_SVF && d.mode > 8) KGPU_THROW(KGPU_ERR_INVALID, "node %u: bad SvfFilterType %u", idx, d.mode);
     if (d.kind == KGPU_ENVELOPE) {
         if (d.n_segments < 1 || !d.segments) KGPU_THROW(KGPU_ERR_INVALID, "node %u: Envelope needs >= 1 segment", idx);
-        if (ki.n_regs > MAX_REGS) KGPU_THROW(KGPU_ERR_UNSUPPORTED, "node %u: Envelope with %u segments is too large", idx, d.n_segments);
+        if (d.n_segments > (uint32_t)(MAX_REGS - REGS_ENVELOPE_BASE) / REGS_ENVELOPE_PER_SEG)
+            KGPU_THROW(KGPU_ERR_UNSUPPORTED, "node %u: Envelope with %u segments is too large (at most %d: %d registers per voice)", idx,
+                       d.n_segments, (MAX_REGS - REGS_ENVELOPE_BASE) / REGS_ENVELOPE_PER_SEG, MAX_REGS);
     }
     if (d.n_wrappers && !d.wrappers) KGPU_THROW(KGPU_ERR_INVALID, "node %u: wrappers pointer is NULL", idx);
     int n_post = 0, n_ar = 0, n_smooth = 0, n_precise = 0;
@@ -843,8 +845,11 @@ void HostPlan::build(const kgpu_graph_desc &d) {
     // (post-mix processing) or when one source feeds many voices: such a source is an internal signal, reduced into its own
     // buffer one level before the voices that read it, and what reads it is cut loose from what produces it -- otherwise
     // the whole bank would be one connected "voice".  Thresholds: a sum of >= mix_min leaves, a node with >= shared_min
-    // consumers.  16 keeps every graph that fitted a voice before (MAX_NODES = 24) exactly as it was; if a component still
-    // outgrows a voice the discovery is repeated with 2 (every fan-in / fan-out point is a cut).
+    // consumers.  16 keeps every graph that fitted a small voice (SMALL_VOICE_NODES) exactly as it was; if a component still
+    // outgrows one the discovery is repeated with 2 (every fan-in / fan-out point is a cut).  Only where neither gives small
+    // voices within the signal budget is a third one tried that cuts a sum only when it has more leaves than one voice can
+    // hold (a master bus over a bank): a voice of up to MAX_NODES nodes then keeps its own partial sums (additive partials).
+    // If that fails too, the first discovery stands, with voices of up to MAX_NODES nodes (a master bus over large voices).
     auto sum_like = [&](int node) {
         if (node < 0) return false;
         const kgpu_node_desc &nd = d.nodes[node];
@@ -972,14 +977,27 @@ void HostPlan::build(const kgpu_graph_desc &d) {
         return largest;
     };
     Discovery D;
-    if (discover(16, 16, D) > (uint32_t)MAX_NODES) {
+    const bool small = discover(16, 16, D) <= (uint32_t)SMALL_VOICE_NODES;
+    bool ok = small && n_outputs + D.n_signals <= 32;
+    if (!small) {
         Discovery D2;
-        bool ok = false;
         try {
-            ok = discover(2, 2, D2) <= (uint32_t)MAX_NODES && n_outputs + D2.n_signals <= 32;
+            ok = discover(2, 2, D2) <= (uint32_t)SMALL_VOICE_NODES && n_outputs + D2.n_signals <= 32;
         } catch (const Error &) {
         }
         if (ok) D = std::move(D2);
+    }
+    if (!ok) {
+        Discovery D3;
+        bool ok3 = false;
+        try {
+            ok3 = discover(MAX_NODES + 1, 16, D3) <= (uint32_t)MAX_NODES && n_outputs + D3.n_signals <= 32;
+        } catch (const Error &) {
+        }
+        if (ok3) D = std::move(D3);
+        // otherwise D stays the first discovery: its voices may now have up to MAX_NODES nodes (compile_template checks).  That is
+        // how a master bus over fewer than MAX_NODES + 1 large voices plans -- the third discovery keeps such a sum whole and
+        // glues the bank into one component, the first cuts it at 16 leaves
     }
     if (n_outputs + D.n_signals > 32)
         KGPU_THROW(KGPU_ERR_UNSUPPORTED, "%u internal signals (sums of voices read by nodes, sources shared between voices): at most %u", D.n_signals, 32 - n_outputs);
@@ -1775,6 +1793,8 @@ struct StreamState {
 #endif
 
 namespace {
+constexpr int NODE_MASK_WORDS = (MAX_NODES + 63) / 64;
+static_assert(MAX_NODES <= 256, "RawEvent::local holds a template node index in a byte");
 // one voice, one launch window: what a separate render call over that window would do
 void simulate_voice_window(HostPlan &P, StreamState &S, StreamState::ThreadCtx &tc, uint32_t gi, uint32_t v, size_t L) {
     Group &g = P.groups[gi];
@@ -1827,11 +1847,12 @@ void simulate_voice_window(HostPlan &P, StreamState &S, StreamState::ThreadCtx &
         // this block's ready events, arrival order
         PROF_T(q0);
         evp.clear();
-        uint32_t mask = 0;
+        // nodes of the voice with a ready event: one bit per template node (MAX_NODES of them)
+        uint64_t mask[NODE_MASK_WORDS] = {};
         while (ei < e1 && ready_block(ei) == b) {
             const RawEvent &r = ev_at(ei++);
             evp.push_back(&r);
-            mask |= 1u << r.local;
+            mask[r.local >> 6] |= 1ull << (r.local & 63u);
         }
         const size_t blk0 = out.size(); // this block's device events: out[blk0 ..)
         PROF_T(q1);
@@ -1839,7 +1860,7 @@ void simulate_voice_window(HostPlan &P, StreamState &S, StreamState::ThreadCtx &
         for (uint32_t li = 0; li < nn; li++) {
             const NodeStatic &ns = g.nstat[li];
             HostNode &hn = g.host[(size_t)v * nn + li];
-            if (!((mask >> li) & 1u) && (ns.fast || !hn.ramp_active)) continue; // (a fast node never ramps: its state is not even touched)
+            if (!((mask[li >> 6] >> (li & 63u)) & 1u) && (ns.fast || !hn.ramp_active)) continue; // (a fast node never ramps: its state is not even touched)
             Sim s{P, sk, li, hn};
             if (ns.fast) {
                 fast_node_block(s, ns, evp.data(), evp.size(), li, block_start);
