@@ -133,7 +133,8 @@ typedef struct {
     uint32_t abi_version;  /* KGPU_ABI_VERSION */
     uint32_t sample_rate;
     uint32_t block_size;
-    uint32_t n_inputs;     /* graph inputs (<= 16): rendered with kgpu_render_inputs; 0: run_without_inputs() */
+    uint32_t n_inputs;     /* graph inputs (<= 65536; at most 16 of them shared, see kgpu_render_inputs): rendered with
+                              kgpu_render_inputs[_device]; 0: run_without_inputs() */
     uint32_t n_outputs;    /* 1..8 */
     int32_t device;        /* CUDA device ordinal, -1 = current */
     uint32_t n_nodes;
@@ -191,9 +192,20 @@ const float *kgpu_output_block(kgpu_plan *plan);
 /* Render n_blocks back to back.  host_out: [n_blocks][n_outputs][block_size] or NULL. */
 int kgpu_render(kgpu_plan *plan, uint64_t n_blocks, float *host_out);
 /* AudioProcessor::run(&[&[F]]) (processor.rs:119-141), batched: the graph's inputs for n_blocks blocks,
- * host_in: [n_blocks][n_inputs][block_size].  A graph with inputs is rendered with this call only (kgpu_render* fail with
- * KGPU_ERR_STATE, like run_without_inputs() asserts inputs() == 0, processor.rs:143); host_out as in kgpu_render. */
+ * host_in: [n_blocks][n_inputs][block_size].  A graph with inputs is rendered with this call or kgpu_render_inputs_device only
+ * (kgpu_render* fail with KGPU_ERR_STATE, like run_without_inputs() asserts inputs() == 0, processor.rs:143); host_out as in
+ * kgpu_render.
+ * An input that only one voice reads (a track through its own effect chain) is a port of that voice: the kernels read it
+ * from the input blocks in place, so a graph may have up to 65536 such inputs.  Any other input -- read by several voices,
+ * summed into a mix or wired straight to an output -- is shared: at most 16 per graph.  host_in is staged launch by launch
+ * through two page-locked buffers of one launch each (a launch's input slice is at most 256 MiB), each copy beside the
+ * previous launch's rendering; host_in is read during the call only. */
 int kgpu_render_inputs(kgpu_plan *plan, uint64_t n_blocks, const float *host_in, float *host_out);
+/* The same with the input blocks already in DEVICE memory on the plan's device (device_in, same layout; read in place, no
+ * copy, and it does not limit the launch length) and the result left in device memory as kgpu_render_device does: enqueued on
+ * `cuda_stream` (NULL = the plan's own stream) without synchronising.  device_in must stay valid until the work has run.
+ * A plan whose voices have ports cannot be sharded over a peer bus (KGPU_ERR_UNSUPPORTED). */
+int kgpu_render_inputs_device(kgpu_plan *plan, uint64_t n_blocks, const float *device_in, float *device_out, void *cuda_stream);
 /* Same, leaving the result in DEVICE memory (device_out: n_blocks*n_outputs*block_size floats
  * on the plan's device) and enqueued on `cuda_stream` (a cudaStream_t, NULL = the plan's own
  * stream) without synchronising: the multi-GPU path reduces the bus from here. */

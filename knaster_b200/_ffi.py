@@ -110,6 +110,7 @@ def lib() -> C.CDLL:
     L.kgpu_render.argtypes = [vp, u64, vp]
     L.kgpu_render_inputs.argtypes = [vp, u64, vp, vp]
     L.kgpu_render_device.argtypes = [vp, u64, vp, vp]
+    L.kgpu_render_inputs_device.argtypes = [vp, u64, vp, vp, vp]
     L.kgpu_plan_synchronize.argtypes = [vp]
     L.kgpu_plan_block_size.argtypes = [vp]
     L.kgpu_plan_block_size.restype = u32
@@ -147,6 +148,7 @@ def lib() -> C.CDLL:
                                       C.POINTER(C.c_size_t), vp, C.POINTER(PlanInfo)]
     L.kgpu_debug_init_reg.argtypes = [C.POINTER(GraphDesc), u32, u32, C.POINTER(u32)]
     L.kgpu_debug_jit_compile.argtypes = [C.POINTER(GraphDesc), u32, C.POINTER(u32), C.POINTER(u32)]
+    L.kgpu_debug_jit_source.argtypes = [C.POINTER(GraphDesc), u32, C.c_char_p, u64, C.POINTER(u64)]
     _lib = L
     return L
 
@@ -230,3 +232,14 @@ def jit_compile(graph, tap_outputs: bool = False):
     a, b = C.c_uint32(0), C.c_uint32(0)
     check(L.kgpu_debug_jit_compile(C.byref(gd), 1 if tap_outputs else 0, C.byref(a), C.byref(b)))
     return a.value, b.value
+
+
+def jit_source(graph, tap_outputs: bool = False) -> List[str]:
+    """Host-only: the CUDA source generated for every voice template of `graph` that has no hand-written recipe (no NVRTC)."""
+    L = lib()
+    gd, _keep = graph_desc(graph)
+    n = C.c_uint64(0)
+    check(L.kgpu_debug_jit_source(C.byref(gd), 1 if tap_outputs else 0, None, 0, C.byref(n)))
+    buf = C.create_string_buffer(n.value)
+    check(L.kgpu_debug_jit_source(C.byref(gd), 1 if tap_outputs else 0, buf, n.value, C.byref(n)))
+    return buf.raw[: n.value].decode().split("\n// ---- end of template\n")[:-1]

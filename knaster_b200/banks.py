@@ -275,6 +275,51 @@ def operator_bank(graph: Graph, n_voices: int, seconds: float, seed: int = 7007,
     return out_ids
 
 
+def input_bank(graph: Graph, n_voices: int, seconds: float, seed: int = 8008, n_notes: int = 8, source: str = "input",
+               stereo: bool = False, only=None, own_outputs: bool = False) -> dict:
+    """One effect chain per track: graph input i -> SvfFilter(Low, per-voice cutoff) -> * EnvAsr.wr_mul(1/N) -> Pan2 -> bus, with
+    `n_notes` notes per voice over `seconds` (any frame of a block).  Each input is read by its own voice only, so it is a port
+    of the one voice template (include/knaster_gpu.h, kgpu_render_inputs).  source="saw": a PolyBlep saw per voice in place
+    of the input (the same bank without input reads).  stereo: voice i filters inputs 2i and 2i + 1 on their own filters
+    and sends them, times the one envelope, to outputs 0 and 1.  only: build just these voices of the bank (the k-th of them
+    reads input k); own_outputs: the k-th voice's Pan2 feeds outputs 2k and 2k + 1 alone.  Returns the node ids per role."""
+    sr = graph.sample_rate
+    n_frames = int(round(seconds * sr))
+    r = _rng(seed)
+    fc = r.uniform(200.0, 8000.0, n_voices)
+    q = r.uniform(0.5, 4.0, n_voices)
+    pan = r.uniform(-1.0, 1.0, n_voices)
+    f0 = 55.0 * 2.0 ** r.uniform(0.0, 5.0, n_voices)
+    att = r.uniform(0.002, 0.05, n_voices)
+    rel = r.uniform(0.05, 0.5, n_voices)
+    on = np.sort(r.integers(0, max(1, n_frames), (n_voices, n_notes)), axis=1)
+    off = on + (r.uniform(0.1, 0.4, (n_voices, n_notes)) * sr).astype(np.int64)
+    ids = {"svf": [], "env": [], "pan": [], "out": []}
+    voices = list(range(n_voices)) if only is None else list(only)
+    with graph.edit() as g:
+        for k, i in enumerate(voices):
+            env = g.push(U.EnvAsr(float(att[i]), float(rel[i])).wr_mul(1.0 / n_voices))
+            if stereo:
+                for c in range(2):
+                    svf = g.push(U.SvfFilter(U.SvfFilterType.Low, float(fc[i]) * (1.0 + 0.1 * c), float(q[i]), 0.0))
+                    sig = g.from_inputs(2 * k + c).to(svf) * env
+                    sig.out([0]).to_graph_out_channels(c)
+                    ids["svf"].append(svf.id()); ids["out"].append(sig._outputs[0][0])
+            else:
+                svf = g.push(U.SvfFilter(U.SvfFilterType.Low, float(fc[i]), float(q[i]), 0.0))
+                src = g.push(U.PolyBlep(U.Waveform.Sawtooth, float(f0[i]))) if source == "saw" else g.from_inputs(k)
+                pn = g.push(U.Pan2(float(pan[i])))
+                sig = (src.to(svf) * env) >> pn
+                if own_outputs:
+                    sig.to_graph_out_channels([2 * k, 2 * k + 1])
+                else:
+                    sig.to_graph_out()
+                ids["svf"].append(svf.id()); ids["pan"].append(pn.id()); ids["out"].append(pn.id())
+            ids["env"].append(env.id())
+    _notes(graph, ids["env"], on[voices], off[voices], n_frames)
+    return ids
+
+
 def bank_builder(workload: str, seconds: float, seed=None):
     """The bench / parity workloads of BASELINE.json by name: returns build(graph, n_voices, voice_offset,
     total_voices) -> one tap node id per voice (the voice's pre-mix signal).  voice_offset / total_voices select a

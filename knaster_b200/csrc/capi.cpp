@@ -118,8 +118,13 @@ struct kgpu_plan {
     DevBuf<float> tap_out;
     // internal signals (plan.hpp HostPlan::signal_level): [signal][frames of the launch], reduced level by level
     DevBuf<float> signals;
-    DevBuf<uint32_t> in_pairs;              // device: (graph input, graph output) pairs wired without a node in between
-    PinBuf<float> in_pinned;                // the caller's input blocks of the current render call
+    DevBuf<uint32_t> in_pairs;              // device: (signal row of a graph input, graph output) pairs wired without a node in between
+    // graph inputs from host memory: a launch's slice [blocks][n_inputs][block_size] goes through one of two page-locked buffers
+    // into one of two device slices, so that the copy of launch L + 1 runs beside the rendering of launch L.  in_copied[b]: the
+    // copy out of buffer b has landed; in_read[b]: the launch that read device slice b is done
+    PinBuf<float> in_pinned[2];
+    DevBuf<float> in_dev[2];
+    cudaEvent_t in_copied[2] = {nullptr, nullptr}, in_read[2] = {nullptr, nullptr};
     DevBuf<uint32_t> sig_which;             // device: the signals of level 0, then level 1, ... (sig_level_off indexes it)
     std::vector<uint32_t> sig_level_off;    // [max_level + 2]
     std::vector<uint32_t> level_rows_end;   // [max_level + 1]: partial rows of the groups up to and including that level
@@ -313,9 +318,10 @@ void prepare_range(kgpu_plan *p, uint64_t n_blocks, uint64_t bpl, cudaStream_t s
     }
 }
 
-uint64_t blocks_per_launch(kgpu_plan *p) {
-    // bound the partial-sum buffer (rows x frames x 4 B) to ~256 MiB
+uint64_t blocks_per_launch(kgpu_plan *p, bool host_inputs) {
+    // bound the partial-sum buffer (rows x frames x 4 B) to ~256 MiB, and so a launch's slice of host input blocks
     uint64_t max_frames = (256ull << 20) / (4ull * std::max(1u, p->n_rows));
+    if (host_inputs && p->host.n_inputs) max_frames = std::min<uint64_t>(max_frames, (256ull << 20) / (4ull * p->host.n_inputs));
     uint64_t bpl = std::max<uint64_t>(1, max_frames / p->host.block_size);
     return std::min<uint64_t>(bpl, p->max_blocks_per_launch);
 }
@@ -390,9 +396,10 @@ void upload_launch_events(kgpu_plan *p, size_t launch, cudaStream_t stream) {
 // device events are already resident and the launches go back to back; otherwise the host half
 // runs launch by launch, one launch ahead of the device: while launch L renders, the control
 // simulation of launch L+1 runs on the host threads and its events are staged in pinned memory.
-// pinned_out: optional page-locked mirror of device_out, filled launch by launch.
+// pinned_out: optional page-locked mirror of device_out, filled launch by launch.  A graph with inputs takes them from host_in
+// (staged launch by launch) or device_in (read in place), [n_blocks][n_inputs][block_size] either way.
 void render_range(kgpu_plan *p, uint64_t n_blocks, float *device_out, cudaStream_t stream, float *pinned_out = nullptr,
-                  const float *host_in = nullptr) {
+                  const float *host_in = nullptr, const float *device_in = nullptr) {
     const uint32_t bs = p->host.block_size, n_out = p->host.n_outputs;
     p->rendered = true;
     const uint64_t total_frames = n_blocks * bs;
@@ -406,7 +413,7 @@ void render_range(kgpu_plan *p, uint64_t n_blocks, float *device_out, cudaStream
         KGPU_THROW(KGPU_ERR_STATE, "kgpu_plan_prepare(%llu) must be followed by a render of %llu blocks, not %llu",
                    (unsigned long long)p->prepared_blocks, (unsigned long long)p->prepared_blocks, (unsigned long long)n_blocks);
     const bool was_prepared = p->prepared;
-    const uint64_t bpl = was_prepared ? p->prepared_bpl : blocks_per_launch(p);
+    const uint64_t bpl = was_prepared ? p->prepared_bpl : blocks_per_launch(p, host_in != nullptr);
     p->prepared = false;
     if (!was_prepared) p->last_h2d_bytes = 0;
     // Streaming path with more than one launch: launch L's mix-bus reduction runs beside launch L+1's rendering, on two
@@ -432,11 +439,21 @@ void render_range(kgpu_plan *p, uint64_t n_blocks, float *device_out, cudaStream
     const bool peer = p->peer_world > 1;
     const uint32_t n_signals = (uint32_t)p->host.signal_level.size();
     const uint32_t n_in = p->host.n_inputs;
-    if (n_in && !host_in) KGPU_THROW(KGPU_ERR_STATE, "this graph has %u inputs: render it with kgpu_render_inputs (AudioProcessor::run), not run_without_inputs", n_in);
-    if (n_in) { // the input blocks, page-locked for the strided copies below
-        p->in_pinned.ensure((size_t)n_blocks * n_in * bs);
-        std::memcpy(p->in_pinned.p, host_in, (size_t)n_blocks * n_in * bs * 4);
+    if (n_in && !host_in && !device_in)
+        KGPU_THROW(KGPU_ERR_STATE, "this graph has %u inputs: render it with kgpu_render_inputs[_device] (AudioProcessor::run), not run_without_inputs", n_in);
+    if (n_in && host_in) {
+        const size_t slice = (size_t)std::min<uint64_t>(bpl, n_blocks) * n_in * bs;
+        if (slice > p->in_dev[0].cap) CUDA_TRY(cudaStreamSynchronize(stream)); // cudaFree of a slice a queued kernel may read
+        ensure_stream_objects(p);
+        for (int b = 0; b < 2; b++) {
+            p->in_pinned[b].ensure(slice);
+            p->in_dev[b].ensure(slice);
+            if (!p->in_copied[b]) CUDA_TRY(cudaEventCreateWithFlags(&p->in_copied[b], cudaEventDisableTiming));
+            if (!p->in_read[b]) CUDA_TRY(cudaEventCreateWithFlags(&p->in_read[b], cudaEventDisableTiming));
+        }
     }
+    if (peer && p->host.has_ports)
+        KGPU_THROW(KGPU_ERR_UNSUPPORTED, "a plan whose voices read graph inputs of their own cannot be sharded over a peer bus");
     if (n_signals) {
         if (peer) KGPU_THROW(KGPU_ERR_UNSUPPORTED, "a plan with internal signals (post-mix nodes, sources shared between voices) cannot be sharded over a peer bus");
         p->signals.ensure((size_t)n_signals * std::min<uint64_t>(bpl, n_blocks) * bs);
@@ -527,10 +544,24 @@ void render_range(kgpu_plan *p, uint64_t n_blocks, float *device_out, cudaStream
                         std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tb).count());
             piece = 0;
         }
-        // graph inputs: [block][input][frame] from the caller -> rows [0, n_inputs) of the signal buffer, [input][frame of the launch]
-        for (uint32_t c = 0; c < n_in; c++)
-            CUDA_TRY(cudaMemcpy2DAsync(p->signals.p + (size_t)c * nf, (size_t)bs * 4, p->in_pinned.p + ((size_t)done * n_in + c) * bs, (size_t)n_in * bs * 4,
-                                       (size_t)bs * 4, (size_t)nb, cudaMemcpyHostToDevice, stream));
+        // graph inputs: this launch's blocks [block][input][frame], in device memory -- the caller's, or a slice staged from the
+        // caller's host buffer through page-locked memory (one copy, beside the previous launch's rendering)
+        const float *in_launch = nullptr;
+        if (n_in && host_in) {
+            const int ib = (int)(launch & 1);
+            const size_t n = (size_t)nb * n_in * bs;
+            if (launch >= 2) CUDA_TRY(cudaEventSynchronize(p->in_copied[ib])); // launch - 2's copy has read the page-locked buffer
+            std::memcpy(p->in_pinned[ib].p, host_in + (size_t)done * n_in * bs, n * 4);
+            if (launch >= 2) CUDA_TRY(cudaStreamWaitEvent(p->h2d_stream, p->in_read[ib], 0)); // ... and its kernels the device slice
+            CUDA_TRY(cudaMemcpyAsync(p->in_dev[ib].p, p->in_pinned[ib].p, n * 4, cudaMemcpyHostToDevice, p->h2d_stream));
+            CUDA_TRY(cudaEventRecord(p->in_copied[ib], p->h2d_stream));
+            CUDA_TRY(cudaStreamWaitEvent(stream, p->in_copied[ib], 0));
+            in_launch = p->in_dev[ib].p;
+        } else if (n_in) in_launch = device_in + (size_t)done * n_in * bs;
+        // shared inputs -> their rows of the signal buffer, [row][frame of the launch]
+        for (uint32_t r = 0; r < (uint32_t)p->host.shared_inputs.size(); r++)
+            CUDA_TRY(cudaMemcpy2DAsync(p->signals.p + (size_t)r * nf, (size_t)bs * 4, in_launch + (size_t)p->host.shared_inputs[r] * bs, (size_t)n_in * bs * 4,
+                                       (size_t)bs * 4, (size_t)nb, cudaMemcpyDeviceToDevice, stream));
         for (uint32_t gi = 0; gi < p->gd.size(); gi++, piece++) {
             Group &g = p->host.groups[gi];
             GroupDev &d = p->gd[gi];
@@ -566,7 +597,8 @@ void render_range(kgpu_plan *p, uint64_t n_blocks, float *device_out, cudaStream
                 }
                 a.scratch = p->scratch.p;
                 if (d.recipe == RECIPE_JIT) {
-                    void *args[] = {&a};
+                    uint32_t n_in_arg = n_in;
+                    void *args[] = {&a, &in_launch, &n_in_arg}; // a template without ports takes the first only
                     CUDA_TRY(cudaLaunchKernel((const void *)d.jit.kernel, dim3((g.n_voices + 31) / 32), dim3(32), args, 0, stream));
                 } else CUDA_TRY(launch_fused(d.recipe, a, stream));
             } else {
@@ -576,6 +608,7 @@ void render_range(kgpu_plan *p, uint64_t n_blocks, float *device_out, cudaStream
                 a.taps = d.taps.p; a.n_taps = (uint32_t)d.host_taps.size(); a.tap_out = p->tap_out.p;
                 a.tap_stride = total_frames; a.tap_frame0 = done * bs; a.sine_table = p->sine.p;
                 a.ext = n_signals ? p->signals.p : nullptr; a.ext_stride = nf;
+                a.in = in_launch; a.n_in = n_in; a.block_size = bs;
                 CUDA_TRY(launch_interp(a, g.prog.n_regs, g.prog.n_slots, stream));
             }
             mark(0, false);
@@ -585,6 +618,7 @@ void render_range(kgpu_plan *p, uint64_t n_blocks, float *device_out, cudaStream
             CUDA_TRY(cudaEventRecord(p->kern_done[launch & 1], stream));
             p->kern_recorded[launch & 1] = true;
         }
+        if (n_in && host_in) CUDA_TRY(cudaEventRecord(p->in_read[launch & 1], stream));
         if (overlap) {
             CUDA_TRY(cudaEventRecord(p->part_ready[pb], stream));
             CUDA_TRY(cudaStreamWaitEvent(rs, p->part_ready[pb], 0));
@@ -750,7 +784,12 @@ void kgpu_plan_destroy(kgpu_plan *p) {
         if (e) cudaEventDestroy(e);
     if (p->h2d_stream) cudaStreamDestroy(p->h2d_stream);
     if (p->d2h_stream) cudaStreamDestroy(p->d2h_stream);
-    p->scratch.release(); p->signals.release(); p->sig_which.release(); p->in_pairs.release(); p->in_pinned.release();
+    p->scratch.release(); p->signals.release(); p->sig_which.release(); p->in_pairs.release();
+    for (int i = 0; i < 2; i++) {
+        p->in_pinned[i].release(); p->in_dev[i].release();
+        if (p->in_copied[i]) cudaEventDestroy(p->in_copied[i]);
+        if (p->in_read[i]) cudaEventDestroy(p->in_read[i]);
+    }
     p->partials.release(); p->row_mask.release(); p->out.release(); p->sine.release(); p->tap_out.release();
     for (cudaEvent_t e : p->kev) cudaEventDestroy(e);
     for (cudaEvent_t e : p->out_ev) cudaEventDestroy(e);
@@ -778,6 +817,19 @@ int kgpu_render_device(kgpu_plan *p, uint64_t n_blocks, float *device_out, void 
         CUDA_TRY(cudaSetDevice(p->device));
         p->timed = true;
         render_range(p, n_blocks, device_out, cuda_stream ? (cudaStream_t)cuda_stream : p->stream);
+        return KGPU_OK;
+    } catch (const Error &e) {
+        return fail(e.code, e.msg);
+    }
+}
+
+int kgpu_render_inputs_device(kgpu_plan *p, uint64_t n_blocks, const float *device_in, float *device_out, void *cuda_stream) {
+    if (!p || !device_out || (p->host.n_inputs && !device_in)) return fail(KGPU_ERR_INVALID, "kgpu_render_inputs_device: NULL argument");
+    if (n_blocks == 0) return KGPU_OK;
+    try {
+        CUDA_TRY(cudaSetDevice(p->device));
+        p->timed = true;
+        render_range(p, n_blocks, device_out, cuda_stream ? (cudaStream_t)cuda_stream : p->stream, nullptr, nullptr, device_in);
         return KGPU_OK;
     } catch (const Error &e) {
         return fail(e.code, e.msg);
@@ -920,7 +972,7 @@ int kgpu_plan_prepare(kgpu_plan *p, uint64_t n_blocks) {
     try {
         CUDA_TRY(cudaSetDevice(p->device));
         if (p->prepared) KGPU_THROW(KGPU_ERR_STATE, "kgpu_plan_prepare: a prepared render is already pending");
-        const uint64_t bpl = blocks_per_launch(p);
+        const uint64_t bpl = blocks_per_launch(p, true); // the render may feed its inputs from host memory
         prepare_range(p, n_blocks, bpl, p->stream);
         CUDA_TRY(cudaStreamSynchronize(p->stream));
         p->prepared = true;
@@ -1471,13 +1523,12 @@ int kgpu_debug_host_bench(const kgpu_graph_desc *desc, const kgpu_event *events,
     }
 }
 
-/* Host-only: generate and compile (NVRTC -> cubin cache, no device needed) the kernel of every voice template of `desc`
- * that has no hand-written recipe.  *n_generated / *n_cached count them; fails with the compiler's log otherwise. */
-int kgpu_debug_jit_compile(const kgpu_graph_desc *desc, uint32_t tap_outputs, uint32_t *n_generated, uint32_t *n_cached) {
-    try {
+} // extern "C"
+// The generated source of every voice template of `desc` that has no hand-written recipe, in group order
+static std::vector<std::string> debug_jit_sources(const kgpu_graph_desc *desc, uint32_t tap_outputs) {
         HostPlan hp;
         hp.build(*desc);
-        uint32_t ng = 0, nc = 0;
+        std::vector<std::string> out;
         for (Group &g : hp.groups) {
             if (match_fused_recipe(g.prog, hp.block_size) >= 0) continue;
             std::vector<uint16_t> tapped;
@@ -1493,8 +1544,19 @@ int kgpu_debug_jit_compile(const kgpu_graph_desc *desc, uint32_t tap_outputs, ui
                     if (std::find(tapped.begin(), tapped.end(), slot) == tapped.end()) tapped.push_back(slot);
                 }
             }
-            const std::string src = jit_source(g.prog, tapped);
-            if (src.empty()) KGPU_THROW(KGPU_ERR_UNSUPPORTED, "jit: the generator does not cover a node of this template");
+            out.push_back(jit_source(g.prog, tapped));
+            if (out.back().empty()) KGPU_THROW(KGPU_ERR_UNSUPPORTED, "jit: the generator does not cover a node of this template");
+        }
+        return out;
+}
+extern "C" {
+
+/* Host-only: generate and compile (NVRTC -> cubin cache, no device needed) the kernel of every voice template of `desc`
+ * that has no hand-written recipe.  *n_generated / *n_cached count them; fails with the compiler's log otherwise. */
+int kgpu_debug_jit_compile(const kgpu_graph_desc *desc, uint32_t tap_outputs, uint32_t *n_generated, uint32_t *n_cached) {
+    try {
+        uint32_t ng = 0, nc = 0;
+        for (const std::string &src : debug_jit_sources(desc, tap_outputs)) {
             std::vector<char> cubin;
             std::string err;
             bool cached = false;
@@ -1504,6 +1566,18 @@ int kgpu_debug_jit_compile(const kgpu_graph_desc *desc, uint32_t tap_outputs, ui
         }
         if (n_generated) *n_generated = ng;
         if (n_cached) *n_cached = nc;
+        return KGPU_OK;
+    } catch (const Error &e) {
+        return fail(e.code, e.msg);
+    }
+}
+
+int kgpu_debug_jit_source(const kgpu_graph_desc *desc, uint32_t tap_outputs, char *buf, uint64_t cap, uint64_t *len) {
+    try {
+        std::string all;
+        for (const std::string &src : debug_jit_sources(desc, tap_outputs)) all += src + "\n// ---- end of template\n";
+        if (len) *len = all.size();
+        if (buf) std::memcpy(buf, all.data(), std::min<uint64_t>(cap, all.size()));
         return KGPU_OK;
     } catch (const Error &e) {
         return fail(e.code, e.msg);

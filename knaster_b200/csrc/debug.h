@@ -30,6 +30,9 @@ int kgpu_debug_host_bench(const kgpu_graph_desc *desc, const kgpu_event *events,
                           uint32_t n_steps, uint32_t n_threads, double *out_ms);
 /* Generate + compile (NVRTC, cubin cache) the kernels of the voice templates of `desc` that have no hand-written recipe. */
 int kgpu_debug_jit_compile(const kgpu_graph_desc *desc, uint32_t tap_outputs, uint32_t *n_generated, uint32_t *n_cached);
+/* The generated CUDA source of the same templates, concatenated, each followed by "\n// ---- end of template\n" (no NVRTC).
+ * Call with buf == NULL for *len; copies at most cap bytes. */
+int kgpu_debug_jit_source(const kgpu_graph_desc *desc, uint32_t tap_outputs, char *buf, uint64_t cap, uint64_t *len);
 /* initial register value of a node register after init() */
 int kgpu_debug_init_reg(const kgpu_graph_desc *desc, uint32_t node, uint32_t reg_offset, uint32_t *value);
 

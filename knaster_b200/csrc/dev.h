@@ -78,6 +78,12 @@ constexpr int MAX_SLOTS = 32;   // live value slots per voice
 // The limits before voices of up to MAX_NODES nodes: a template inside all three is "small".  Voice discovery keeps cutting
 // the graph where it did for such voices, and the interpreter keeps their chunk, so graphs that fitted them plan as before.
 constexpr int SMALL_VOICE_NODES = 24, SMALL_VOICE_REGS = 192, SMALL_VOICE_SLOTS = 24;
+// Ports: graph inputs that only one voice reads (a track through its own effect chain).  A node reads port k of its template
+// through in_slot / ar_slot SLOT_PORT0 + k -- below the codes of internal signals (-2 - signal, signal < 32) -- and which input
+// that is, is per voice: register DevProgram::port_reg + k holds the voice's input channel.
+constexpr int MAX_PORTS = 4;
+constexpr int SLOT_PORT0 = -32768;
+constexpr int SLOT_PORT_END = SLOT_PORT0 + MAX_PORTS; // slot < SLOT_PORT_END: a port
 
 struct DevNode {
     uint8_t kind, mode, n_in, n_out;
@@ -99,7 +105,7 @@ struct DevProgram {
     uint16_t ubus_slot[MAX_BUS];   // value slot of each
     uint32_t ubus_mask[MAX_BUS];   // graph output channels each one feeds (stereo .out([0,0]) => 0b11)
     float sample_rate;             // F::new(sr as f32)
-    float _pad;
+    uint16_t n_ports, port_reg;    // ports of the template and the first of their n_ports registers (after every node's)
     double sinwt_k;                // TABLE_SIZE * FRACTIONAL_PART * (1 / sr)   osc.rs:144-145
     DevNode nodes[MAX_NODES];
 };

@@ -118,8 +118,11 @@ __global__ void __launch_bounds__(32) render_interp(InterpArgs a) {
     }
     L.fetch();
 
+    const uint32_t port_reg = prog->port_reg;
     for (uint32_t c0 = 0; c0 < a.n_frames; c0 += CH) {
         const uint32_t nf = min(CH, a.n_frames - c0);
+        // a chunk lies inside one block (CH divides the block size): port k reads a.in[in_c0 + channel_k * block_size + f]
+        const size_t in_c0 = a.in ? (size_t)(c0 / a.block_size) * a.n_in * a.block_size + c0 % a.block_size : 0;
         for (uint32_t n = 0; n < n_nodes; n++) {
             const DevNode &dn = prog->nodes[n];
             const bool evc = __any_sync(0xFFFFFFFFu, L.next_node == n && L.next_frame < c0 + nf);
@@ -157,9 +160,12 @@ __global__ void __launch_bounds__(32) render_interp(InterpArgs a) {
         _Pragma("unroll") for (int k = 0; k < 16; k++) y_[k] = (EXPR_);                \
         _Pragma("unroll") for (int k = 0; k < 16; k++) sval[(o0_ * CH + g0_ + k) * 32] = y_[k] * g_; \
     }
-// the value a node reads: a value slot of the voice (>= 0), the permanent zero channel (-1), or an internal signal of the plan
-// (<= -2: sums of voices read by nodes, sources shared between voices -- a.ext[signal][frame of the launch], the same for every voice)
-#define RDV(slot_, f_) ((slot_) >= 0 ? sval[((slot_) * CH + (f_)) * 32] : ((slot_) == -1 ? 0.f : a.ext[(size_t)(-2 - (slot_)) * a.ext_stride + c0 + (f_)]))
+// the value a node reads: a value slot of the voice (>= 0), the permanent zero channel (-1), an internal signal of the plan
+// (<= -2: sums of voices read by nodes, sources shared between voices -- a.ext[signal][frame of the launch], the same for every
+// voice), or a port (< SLOT_PORT_END: the graph input whose channel the voice holds in register port_reg + port)
+#define RDV(slot_, f_) ((slot_) >= 0 ? sval[((slot_) * CH + (f_)) * 32] : ((slot_) == -1 ? 0.f : (slot_) >= SLOT_PORT_END            \
+    ? a.ext[(size_t)(-2 - (slot_)) * a.ext_stride + c0 + (f_)]                                                                      \
+    : __ldg(a.in + in_c0 + (size_t)sreg[(port_reg + (uint32_t)((slot_) - SLOT_PORT0)) * 32] * a.block_size + (f_))))
 #define LOAD16(x_, slot_)                                                              \
     float x_[16];                                                                      \
     _Pragma("unroll") for (int k = 0; k < 16; k++) x_[k] = RDV(slot_, g0_ + k);

@@ -26,6 +26,8 @@ struct InterpArgs {
     const float *sine_table; // device, 16384 f32 (wavetable.rs:130-139)
     const float *ext;        // internal signals [signal][ext_stride] of this launch; NULL if none
     uint32_t ext_stride;
+    const float *in;         // ports (dev.h): the caller's input blocks [block][n_in][block_size] from the launch's first block
+    uint32_t n_in, block_size;
 };
 
 cudaError_t launch_interp(const InterpArgs &a, uint32_t n_regs, uint32_t n_slots, cudaStream_t stream);

@@ -677,6 +677,19 @@ void compile_template(Group &g, uint32_t sample_rate, const std::vector<std::pai
             dn.n_ar++;
         }
     }
+    // ports: one register each after every node's, holding the voice's input channel
+    uint32_t n_ports = 0;
+    for (const TemplateNode &tn : t.nodes) {
+        for (auto &e : tn.in)
+            if (is_port_src(e.first)) n_ports = std::max(n_ports, (uint32_t)(e.first - PORT_SRC0) + 1);
+        for (auto &pe : tn.par)
+            if (is_port_src(std::get<1>(pe))) n_ports = std::max(n_ports, (uint32_t)(std::get<1>(pe) - PORT_SRC0) + 1);
+    }
+    if (n_ports > (uint32_t)MAX_PORTS)
+        KGPU_THROW(KGPU_ERR_UNSUPPORTED, "a voice reads %u graph inputs that no other voice reads (limit %d per voice)", n_ports, MAX_PORTS);
+    p.n_ports = (uint16_t)n_ports;
+    p.port_reg = (uint16_t)(n_ports ? std::min<uint32_t>(reg, 0xFFFF) : 0u);
+    reg += n_ports;
     if (reg > (uint32_t)MAX_REGS) KGPU_THROW(KGPU_ERR_UNSUPPORTED, "voice needs %u registers (limit %d)", reg, MAX_REGS);
     p.n_regs = reg;
     // value slots: liveness-based reuse, the analogue of allocate_node_buffers (graph.rs:1588-1704)
@@ -702,7 +715,8 @@ void compile_template(Group &g, uint32_t sample_rate, const std::vector<std::pai
         for (int c = 0; c < MAX_IN; c++) dn.in_slot[c] = -1;
         for (size_t c = 0; c < tn.in.size(); c++) {
             auto &e = tn.in[c];
-            if (e.first <= EXT_BASE) dn.in_slot[c] = (int16_t)e.first; // an internal signal, read from its buffer
+            if (e.first <= EXT_BASE) // an internal signal, read from its buffer, or a port
+                dn.in_slot[c] = (int16_t)(is_port_src(e.first) ? SLOT_PORT0 + (e.first - PORT_SRC0) : e.first);
             if (e.first < 0) continue;
             dn.in_slot[c] = (int16_t)g.slot_of[e.first][e.second];
             if (last_use[e.first][e.second] == (int)i) dying.push_back(e);
@@ -713,8 +727,8 @@ void compile_template(Group &g, uint32_t sample_rate, const std::vector<std::pai
         for (auto &pe : tn.par) {
             int src = std::get<1>(pe);
             uint32_t ch = std::get<2>(pe);
-            if (src <= EXT_BASE) { // routed from an internal signal
-                if (has_ar) dn.ar_slot[ai++] = (int16_t)src;
+            if (src <= EXT_BASE) { // routed from an internal signal or a port
+                if (has_ar) dn.ar_slot[ai++] = (int16_t)(is_port_src(src) ? SLOT_PORT0 + (src - PORT_SRC0) : src);
                 continue;
             }
             if (has_ar) dn.ar_slot[ai++] = (int16_t)g.slot_of[src][ch];
@@ -766,9 +780,11 @@ void HostPlan::build(const kgpu_graph_desc &d) {
     if (d.sample_rate == 0 || d.block_size == 0) KGPU_THROW(KGPU_ERR_INVALID, "sample_rate and block_size must be non-zero"); // processor.rs:75
     if (d.block_size > 65535) KGPU_THROW(KGPU_ERR_INVALID, "block_size must fit the u16 in-block delay (graph_gen.rs:292)");
     if (d.n_outputs < 1 || d.n_outputs > (uint32_t)MAX_BUS) KGPU_THROW(KGPU_ERR_UNSUPPORTED, "n_outputs must be 1..%d", MAX_BUS);
-    if (d.n_inputs > 16) KGPU_THROW(KGPU_ERR_UNSUPPORTED, "more than 16 graph inputs");
+    if (d.n_inputs > MAX_GRAPH_INPUTS) KGPU_THROW(KGPU_ERR_UNSUPPORTED, "%u graph inputs: at most %u", d.n_inputs, MAX_GRAPH_INPUTS);
     n_inputs = d.n_inputs;
     input_to_output.clear();
+    shared_inputs.clear();
+    has_ports = false;
     if ((d.n_nodes && !d.nodes) || (d.n_edges && !d.edges) || (d.n_param_edges && !d.param_edges))
         KGPU_THROW(KGPU_ERR_INVALID, "NULL array in graph description");
     sample_rate = d.sample_rate;
@@ -976,13 +992,44 @@ void HostPlan::build(const kgpu_graph_desc &d) {
             if (D.comp[i] >= 0) largest = std::max(largest, ++size[find(D.comp[i])]);
         return largest;
     };
+    // Graph inputs after a discovery: owner[i] = the component of the one voice that reads input i (a port of its template), -1
+    // for a shared input (read by several voices, summed into a mix, wired to an output), -2 for one nothing reads.  Returns the
+    // number of shared inputs: only they take signal rows.
+    auto classify_inputs = [&](const Discovery &D, std::vector<int> &owner) -> uint32_t {
+        owner.assign(n_inputs, -2);
+        auto root = [&](int x) {
+            while (D.uf[x] != x) x = D.uf[x];
+            return x;
+        };
+        auto read = [&](uint32_t in, uint32_t nk) {
+            const int c = root(D.comp[nk]);
+            owner[in] = owner[in] == -2 || owner[in] == c ? c : -1;
+        };
+        for (uint32_t nk = 0; nk < N; nk++) {
+            if (D.comp[nk] < 0) continue;
+            for (uint32_t k = in_off[nk]; k < in_off[nk + 1]; k++)
+                if (in_edges[k].first == KGPU_GRAPH) read(in_edges[k].second, nk);
+            for (auto &pe : par_edges[nk])
+                if (std::get<1>(pe) == KGPU_GRAPH) read(std::get<2>(pe), nk);
+        }
+        for (const Leaf &lf : D.leaves)
+            if (lf.node == KGPU_GRAPH) owner[lf.ch] = -1;
+        uint32_t n_shared = 0;
+        for (int o : owner) n_shared += o == -1;
+        return n_shared;
+    };
+    // outputs + shared inputs + internal signals within the 32 rows of the partial-sum masks
+    auto signals_fit = [&](const Discovery &D) {
+        std::vector<int> owner;
+        return n_outputs + classify_inputs(D, owner) + (D.n_signals - n_inputs) <= 32;
+    };
     Discovery D;
     const bool small = discover(16, 16, D) <= (uint32_t)SMALL_VOICE_NODES;
-    bool ok = small && n_outputs + D.n_signals <= 32;
+    bool ok = small && signals_fit(D);
     if (!small) {
         Discovery D2;
         try {
-            ok = discover(2, 2, D2) <= (uint32_t)SMALL_VOICE_NODES && n_outputs + D2.n_signals <= 32;
+            ok = discover(2, 2, D2) <= (uint32_t)SMALL_VOICE_NODES && signals_fit(D2);
         } catch (const Error &) {
         }
         if (ok) D = std::move(D2);
@@ -991,7 +1038,7 @@ void HostPlan::build(const kgpu_graph_desc &d) {
         Discovery D3;
         bool ok3 = false;
         try {
-            ok3 = discover(MAX_NODES + 1, 16, D3) <= (uint32_t)MAX_NODES && n_outputs + D3.n_signals <= 32;
+            ok3 = discover(MAX_NODES + 1, 16, D3) <= (uint32_t)MAX_NODES && signals_fit(D3);
         } catch (const Error &) {
         }
         if (ok3) D = std::move(D3);
@@ -999,8 +1046,36 @@ void HostPlan::build(const kgpu_graph_desc &d) {
         // how a master bus over fewer than MAX_NODES + 1 large voices plans -- the third discovery keeps such a sum whole and
         // glues the bank into one component, the first cuts it at 16 leaves
     }
+    // shared inputs become signal rows 0 .. n_shared - 1, the internal signals follow; a port edge is marked -2 - input
+    std::vector<int> owner;
+    const uint32_t n_shared = classify_inputs(D, owner);
+    if (n_shared > (uint32_t)MAX_SHARED_INPUTS)
+        KGPU_THROW(KGPU_ERR_UNSUPPORTED, "%u graph inputs are shared (read by more than one voice, summed into a mix or wired to an output): at most %d",
+                   n_shared, MAX_SHARED_INPUTS);
+    {
+        std::vector<int> remap(D.n_signals);
+        for (uint32_t i = 0; i < n_inputs; i++) {
+            if (owner[i] >= 0) {
+                remap[i] = -2 - (int)i;
+                has_ports = true;
+            } else if (owner[i] == -1) {
+                remap[i] = (int)shared_inputs.size();
+                shared_inputs.push_back(i);
+            }
+        }
+        for (uint32_t sg = n_inputs; sg < D.n_signals; sg++) remap[sg] = (int)(n_shared + sg - n_inputs);
+        for (int &e : D.in_ext)
+            if (e >= 0) e = remap[e];
+        for (auto &pl : D.par_ext)
+            for (int &e : pl)
+                if (e >= 0) e = remap[e];
+        for (Leaf &lf : D.leaves)
+            if (lf.target >= n_outputs) lf.target = n_outputs + (uint32_t)remap[lf.target - n_outputs];
+        D.n_signals = n_shared + (D.n_signals - n_inputs);
+    }
     if (n_outputs + D.n_signals > 32)
-        KGPU_THROW(KGPU_ERR_UNSUPPORTED, "%u internal signals (sums of voices read by nodes, sources shared between voices): at most %u", D.n_signals, 32 - n_outputs);
+        KGPU_THROW(KGPU_ERR_UNSUPPORTED, "%u internal signals (sums of voices read by nodes, sources shared between voices, shared graph inputs): at most %u",
+                   D.n_signals, 32 - n_outputs);
     n_mix_nodes = D.n_mix;
     std::vector<Leaf> &leaves = D.leaves;
     std::vector<int> &comp = D.comp;
@@ -1014,7 +1089,8 @@ void HostPlan::build(const kgpu_graph_desc &d) {
     for (auto &lf : leaves) {
         if (lf.node == KGPU_GRAPH) {
             if (lf.target >= n_outputs) KGPU_THROW(KGPU_ERR_UNSUPPORTED, "a graph input summed into an internal mix is not supported");
-            input_to_output.push_back({lf.ch, lf.target});
+            const uint32_t row = (uint32_t)(std::lower_bound(shared_inputs.begin(), shared_inputs.end(), lf.ch) - shared_inputs.begin());
+            input_to_output.push_back({row, lf.target});
             continue;
         }
         int c = find(comp[lf.node]);
@@ -1047,7 +1123,7 @@ void HostPlan::build(const kgpu_graph_desc &d) {
             state[c] = 1;
             int lv = 0;
             for (int sg : reads[c]) {
-                if ((uint32_t)sg < n_inputs) continue; // a graph input: there before the first launch
+                if ((uint32_t)sg < n_shared) continue; // a graph input: there before the first launch
                 int sl = 0;
                 for (int f : feeders[sg]) sl = std::max(sl, level_of(f));
                 signal_level[sg] = std::max(signal_level[sg], sl);
@@ -1058,7 +1134,7 @@ void HostPlan::build(const kgpu_graph_desc &d) {
         };
         max_level = 0;
         for (int c : comp_order) max_level = std::max(max_level, level_of(c));
-        for (uint32_t sg = n_inputs; sg < D.n_signals; sg++)
+        for (uint32_t sg = n_shared; sg < D.n_signals; sg++)
             if (signal_level[sg] < 0) { // a signal nobody reads cannot exist; keep it well-defined anyway
                 int sl = 0;
                 for (int f : feeders[sg]) sl = std::max(sl, comp_level[f]);
@@ -1109,6 +1185,13 @@ void HostPlan::build(const kgpu_graph_desc &d) {
         Template t;
         t.level = comp_level[c];
         t.nodes.resize(order.size());
+        std::vector<uint32_t> ports; // the graph input of each port, in the order the template first reads them
+        auto port_src = [&](int ext) {
+            const uint32_t in = (uint32_t)(-2 - ext);
+            size_t k = std::find(ports.begin(), ports.end(), in) - ports.begin();
+            if (k == ports.size()) ports.push_back(in);
+            return PORT_SRC0 + (int)k;
+        };
         for (size_t li = 0; li < order.size(); li++) {
             uint32_t nk = order[li];
             const kgpu_node_desc &nd = d.nodes[nk];
@@ -1118,11 +1201,13 @@ void HostPlan::build(const kgpu_graph_desc &d) {
             tn.wrappers.assign(nd.wrappers, nd.wrappers + nd.n_wrappers);
             for (uint32_t k = in_off[nk]; k < in_off[nk + 1]; k++) {
                 if (D.in_ext[k] >= 0) tn.in.push_back({EXT_BASE - D.in_ext[k], 0u});
+                else if (D.in_ext[k] <= -2) tn.in.push_back({port_src(D.in_ext[k]), 0u});
                 else tn.in.push_back({in_edges[k].first >= 0 ? local_of[in_edges[k].first] : -1, in_edges[k].second});
             }
             for (size_t k = 0; k < par_edges[nk].size(); k++) {
                 auto &pe = par_edges[nk][k];
                 if (D.par_ext[nk][k] >= 0) tn.par.push_back({std::get<0>(pe), EXT_BASE - D.par_ext[nk][k], 0u});
+                else if (D.par_ext[nk][k] <= -2) tn.par.push_back({std::get<0>(pe), port_src(D.par_ext[nk][k]), 0u});
                 else tn.par.push_back({std::get<0>(pe), local_of[std::get<1>(pe)], std::get<2>(pe)});
             }
         }
@@ -1141,6 +1226,7 @@ void HostPlan::build(const kgpu_graph_desc &d) {
         Group &g = groups[gi];
         uint32_t voice = g.n_voices++;
         g.voice_nodes.push_back(order);
+        g.port_input.insert(g.port_input.end(), ports.begin(), ports.end());
         for (size_t li = 0; li < order.size(); li++) {
             node_ref[order[li]].group = gi;
             node_ref[order[li]].voice = voice;
@@ -1217,6 +1303,8 @@ void HostPlan::build(const kgpu_graph_desc &d) {
             if (getenv("KGPU_HOST_GENERIC")) ns.fast = false; // tests: the block-by-block model for every node
         }
         auto R = [&](uint32_t reg, uint32_t v) -> uint32_t & { return g.init_regs[(size_t)reg * V + v]; };
+        for (uint32_t v = 0; v < V; v++)
+            for (uint32_t k = 0; k < g.prog.n_ports; k++) R(g.prog.port_reg + k, v) = g.port_input[(size_t)v * g.prog.n_ports + k];
         for (uint32_t v = 0; v < V; v++)
             for (uint32_t li = 0; li < nn; li++) {
                 const kgpu_node_desc &nd = d.nodes[g.voice_nodes[v][li]];

@@ -144,8 +144,13 @@ struct Template {
     int level = 0;                                           // 0: reads no internal signal; else 1 + the highest level it reads
     bool same_shape(const Template &o) const;
 };
-// an input / parameter-route source that is not a node of the same voice: internal signal s is encoded as EXT_BASE - s
+// an input / parameter-route source that is not a node of the same voice: internal signal s is encoded as EXT_BASE - s,
+// port k of the template (a graph input only this voice reads, dev.h) as PORT_SRC0 + k
 constexpr int EXT_BASE = -2;
+constexpr int PORT_SRC0 = -(1 << 30);
+constexpr uint32_t MAX_GRAPH_INPUTS = 65536;
+constexpr int MAX_SHARED_INPUTS = 16; // graph inputs that are not ports: each takes a signal row
+inline bool is_port_src(int src) { return src < PORT_SRC0 / 2; }
 
 struct Group {
     Template tpl;
@@ -156,6 +161,7 @@ struct Group {
     std::vector<HostNode, HugeAllocator<HostNode>> host; // [voice * n_nodes + local]
     std::vector<NodeStatic> nstat;                  // [local]
     std::vector<std::vector<uint16_t>> slot_of;     // [local][channel] -> value slot
+    std::vector<uint32_t> port_input;               // [voice * prog.n_ports + port] -> graph input (init_regs holds it too)
     int fused_recipe = -1;                          // index into the fused-kernel table, -1 = interpreter
     std::string kernel_name;
 };
@@ -222,12 +228,16 @@ struct HostPlan {
     // (one LFO into every voice's cutoff).  Each is rendered like a graph output -- its contributors' partial rows are
     // reduced into a buffer [signal][frame] -- one level before the voices that read it.  signal_level[s] = the level of
     // its highest contributor; groups are sorted by level.
-    // The graph's own inputs (AudioProcessor::run(&[&[F]]), processor.rs:119-141) are the first n_inputs signals, level -1:
-    // the caller's input block is copied into their rows before a launch.
+    // The graph's own inputs (AudioProcessor::run(&[&[F]]), processor.rs:119-141) are of two sorts.  One that a single voice
+    // reads is a port of that voice's template (dev.h): the kernels read it from the caller's input blocks in place.  Every other
+    // one -- read by several voices, summed into a mix, wired to an output -- is shared: the first shared_inputs.size() signals,
+    // level -1, whose rows are copied from the caller's input blocks before a launch.
     std::vector<int> signal_level;
     int max_level = 0;
     uint32_t n_inputs = 0;
-    std::vector<std::pair<uint32_t, uint32_t>> input_to_output; // graph input wired (or summed) straight into a graph output
+    std::vector<uint32_t> shared_inputs;                        // [signal row] -> graph input
+    bool has_ports = false;
+    std::vector<std::pair<uint32_t, uint32_t>> input_to_output; // (signal row of a graph input, graph output) wired or summed straight
     uint64_t graph_hash = 0;       // of the whole graph description (snapshots only restore into the same graph)
     uint64_t dropped_changes = 0, ignored_delays = 0, device_events = 0;
     std::vector<RawEvent, DefaultInitAllocator<RawEvent>> pending; // not yet simulated, arrival order

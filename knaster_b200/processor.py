@@ -140,7 +140,7 @@ class AudioProcessor:
     # -- batched rendering
     def render(self, n_blocks: int, out: Optional[np.ndarray] = None, inputs: Optional[np.ndarray] = None) -> np.ndarray:
         """Render n_blocks; returns host audio [n_blocks][outputs][block_size].  inputs: [n_blocks][graph inputs][block_size]
-        for a graph with inputs (the batched form of ``run``)."""
+        for a graph with inputs (the batched form of ``run``), streamed to the device launch by launch."""
         self._ensure_plan()
         self._push_events()
         self._started = True
@@ -158,13 +158,19 @@ class AudioProcessor:
         self._last_render_frames = n_blocks * self.block_size()
         return out
 
-    def render_device(self, n_blocks: int, device_ptr: int, stream: int = 0) -> None:
+    def render_device(self, n_blocks: int, device_ptr: int, stream: int = 0, inputs_device_ptr: Optional[int] = None) -> None:
         """Render into device memory (n_blocks*outputs*block_size floats at device_ptr), enqueued
-        on `stream` (cudaStream_t as int, 0 = the plan's own stream), without synchronising."""
+        on `stream` (cudaStream_t as int, 0 = the plan's own stream), without synchronising.
+        inputs_device_ptr: for a graph with inputs, its input blocks in device memory, [n_blocks][graph inputs][block_size] f32,
+        read in place (they must stay valid until the render has run)."""
         self._ensure_plan()
         self._push_events()
         self._started = True
-        _ffi.check(self._lib.kgpu_render_device(self._plan, n_blocks, C.c_void_p(device_ptr), C.c_void_p(stream)))
+        if inputs_device_ptr is not None:
+            _ffi.check(self._lib.kgpu_render_inputs_device(self._plan, n_blocks, C.c_void_p(inputs_device_ptr), C.c_void_p(device_ptr),
+                                                           C.c_void_p(stream)))
+        else:
+            _ffi.check(self._lib.kgpu_render_device(self._plan, n_blocks, C.c_void_p(device_ptr), C.c_void_p(stream)))
         self._last_render_frames = n_blocks * self.block_size()
 
     def synchronize(self) -> None:

@@ -37,6 +37,8 @@ extern "C" {
     pub fn kgpu_render(plan: *mut kgpu_plan, n_blocks: u64, host_out: *mut f32) -> c_int;
     pub fn kgpu_render_inputs(plan: *mut kgpu_plan, n_blocks: u64, host_in: *const f32, host_out: *mut f32) -> c_int;
     pub fn kgpu_render_device(plan: *mut kgpu_plan, n_blocks: u64, device_out: *mut f32, cuda_stream: *mut c_void) -> c_int;
+    pub fn kgpu_render_inputs_device(plan: *mut kgpu_plan, n_blocks: u64, device_in: *const f32, device_out: *mut f32,
+                                     cuda_stream: *mut c_void) -> c_int;
     pub fn kgpu_plan_prepare(plan: *mut kgpu_plan, n_blocks: u64) -> c_int;
     pub fn kgpu_plan_synchronize(plan: *mut kgpu_plan) -> c_int;
     pub fn kgpu_plan_block_size(plan: *const kgpu_plan) -> u32;
